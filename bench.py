@@ -1,6 +1,7 @@
 """bench.py -- scheduling decisions/sec of the batched env on N B200s (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--configs C3,C4,C5|none]
+                    [--dump-outputs DIR]
 
 Headline (the JSON line's top-level keys) = BASELINE.json configs[1], "C2": 4096 environments per GPU, 50 jobs x 10
 executors, fair scheduler (RoundRobinScheduler(10, dynamic_partition=True)), synthetic TPC-H-shaped bank (SURVEY.md
@@ -17,6 +18,8 @@ included).
              itself) / its CUDA-event duration, against MEASURED_PEAKS.json
   cpu_baseline : the C oracle port (oracle/sim_oracle.c) on the box's host cores, same workload
   --impl reference : only that CPU arm, as its own JSON line
+  --dump-outputs DIR : after the headline's timed steps, what a caller of the fused rollout holds after the last of them
+             (dump_outputs), as DIR/<name>.npy; inputs depend on the arguments only, so two builds can be compared
 
 "configs" (same JSON line) carries short runs of the other BASELINE.json configurations, each with its own value,
 roofline, cpu_baseline and e2e:
@@ -355,6 +358,48 @@ def timed_fair_rollouts(cx, env, seeds, seed_step, W, K, D, pre_decisions=0):
     return kern_ms, env.stats(), launches, stats[K - 1], t_wall
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(env, rollout_stats, out_dir: str, limit: int = DUMP_LIMIT) -> list[str]:
+    """Writes what a caller of the fused rollout holds after it, as out_dir/<name>.npy: every field of the observation
+    headers (reward, wall_time, num_nodes, ...), the observation graphs (nodes, edge_links, dag_ptr, exec_supplies: the
+    valid rows of each env, concatenated in env order; the header counts split them), the per-env counters since the
+    last reset_stats (stats_<field>) and `rollout_stats`, the collect_stats vector as the caller holds it (with several
+    ranks: after the all-reduce, i.e. summed over all ranks, while the other files hold this rank's envs).  Only
+    float32 / float64 files: integers are stored as float64 (exact below 2**53).  If all envs at their buffer
+    capacities do not fit in `limit` bytes, a fixed sample of them (numpy seed 0) is written, in env order; env_ids
+    lists the envs written.  Which envs are written depends on the env count and capacities only, never on what the
+    rollout computed, so two builds are compared on the same envs.  Returns the names written."""
+    import torch
+
+    from spark_sched_sim_b200 import _native as nat
+
+    h = env.hdr()
+    B = len(h)
+    n, m, j = (h[f].astype(np.int64) for f in ("num_nodes", "num_edges", "num_active_jobs"))
+    S, M, J = env.node_stride, env.edge_stride, env.job_stride
+    per_env = 8 * (len(h.dtype.names) + len(nat.STATS_FIELDS) + 1) + 12 * S + 16 * M + 8 * (J + 1) + 8 * J
+    fit = (limit - (8 << 10)) // per_env  # less the fixed-size rollout_stats and the .npy headers
+    envs = np.arange(B) if fit >= B else np.sort(np.random.default_rng(0).permutation(B)[:fit])
+
+    def rows(view, count):
+        a = view[torch.as_tensor(envs, device=view.device)].cpu().numpy()
+        return a[np.arange(a.shape[1])[None, :] < count[envs, None]]
+
+    out = {f: h[f][envs] for f in h.dtype.names}
+    out.update(nodes=rows(env.nodes, n), edge_links=rows(env.edge_links, m), dag_ptr=rows(env.dag_ptr, j + 1),
+               exec_supplies=rows(env.exec_supplies, j))
+    st = env.stats_per_env()
+    out.update({f"stats_{f}": st[f][envs] for f in nat.STATS_FIELDS})
+    out["rollout_stats"] = rollout_stats.cpu().numpy()
+    out["env_ids"] = envs
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(osp.join(out_dir, name + ".npy"), v if v.dtype in (np.float32, np.float64) else v.astype(np.float64))
+    return sorted(out)
+
+
 def e2e_step_loop(cx, cfg, seeds, seed_step, Ke, De, budget, with_obs):
     """The caller-facing loop of a vector env through the host-buffer C ABI; with_obs: also the packed observation
     graphs of all envs every call."""
@@ -418,6 +463,8 @@ def run_c2(cx, args):
         sampler.start()
     kern_ms, st, launches, stats_vec, t_wall = timed_fair_rollouts(cx, env, seeds, seed_step, W, K, D)
     clocks = sampler.stop() if cx.rank == 0 else None
+    if args.dump_outputs and cx.rank == 0:
+        dump_outputs(env, stats_vec, args.dump_outputs)
     n_err = int((env.hdr()["error"] != 0).sum())
     max_ms, (total_dec, total_ev, total_eps, total_err) = reduce_max_sum(
         cx, kern_ms, [st["decisions"], st["events"], st["episodes"], n_err])
@@ -657,7 +704,9 @@ def run_decima(cx, args, with_update: bool):
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline; the extra configs and the e2e loops run their own short "
+                         "windows (2 .. 5 steps), each reported in its entry")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--envs", type=int, default=ENVS_PER_GPU)
@@ -668,7 +717,14 @@ def main() -> None:
     ap.add_argument("--configs", default="C3,C4,C5", help="extra BASELINE.json configurations to run (or 'none')")
     ap.add_argument("--c3-envs", type=int, default=C3_ENVS)
     ap.add_argument("--c4-envs", type=int, default=C4_ENVS)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline's outputs after its last timed step to DIR/<name>.npy (rank 0's envs; "
+                         "rollout_stats is the all-reduced sum over the ranks)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm has none")
     if args.impl == "reference":
         run_reference(args)
         return

@@ -6,8 +6,8 @@ compatibility layer for callers that drive the gym facade step by step.
 The reference walks the jobs and their nodes in Python loops.  Here one vectorised pass (`job_choices`) answers
 "which `stage_idx` would this job get" for every active job at once -- segment minima over the observation's node
 arrays -- and the policies are a few array expressions on top of it.  `tests/test_host_schedulers.py` pins the
-classes to the actions the reference recorded and, where `/root/reference` exists, to the reference's own classes
-run side by side on the same observations."""
+classes to the actions the reference recorded and to what the reference's classes return and leave in the
+observation dict on the same observations (tests/golden/scheduler_vectors.npz)."""
 from __future__ import annotations
 
 import numpy as np

@@ -13,7 +13,8 @@ GOLDEN_DIR = osp.join(osp.dirname(osp.abspath(__file__)), "golden")
 def golden_names(slim=None):
     names = sorted(osp.basename(p)[:-4] for p in glob.glob(osp.join(GOLDEN_DIR, "*.npz")))
     # fixtures that are not traces
-    names = [n for n in names if n not in ("decima_model", "learner_vectors") and not n.startswith("decima_grads_")]
+    names = [n for n in names if n not in ("decima_model", "learner_vectors", "scheduler_vectors")
+             and not n.startswith("decima_grads_")]
     if slim is None:
         return names
     return [n for n in names if n.startswith(("c2_", "c4_", "decima_c2_", "decima_c3_")) == slim]
