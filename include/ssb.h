@@ -219,7 +219,10 @@ int ssb_packed_obs_bytes(ssb_env *env, size_t *bytes);
 int ssb_get_obs_host(ssb_env *env, ssb_packed_obs *out, void *scratch, size_t scratch_bytes);
 
 /* fused rollout: every env takes `num_decisions` decisions with the built-in fair (dynamic_partition
- * = 1) or FIFO (= 0) policy (round_robin.py:14-49) evaluated on the observation it just wrote.
+ * = 1) or FIFO (= 0) policy (round_robin.py:14-49), which reads the simulator state directly.
+ * The intermediate observation graphs are not materialised: when the call returns, the views hold the
+ * observation that is live then (header, graph and reward), and the ssb_stats counters count every
+ * observation.  Per-decision rewards are available through ssb_rollout_fair_traj.
  * auto_reset != 0: a finished env re-seeds itself with seed + seed_step * reset_count
  * (rollout_worker.py:118-120) and continues; otherwise it idles once done. */
 int ssb_rollout_fair(ssb_env *env, int32_t num_decisions, int32_t dynamic_partition, int32_t auto_reset,

@@ -27,7 +27,8 @@ from spark_sched_sim_b200.batched_env import BatchedSparkSchedSimEnv  # noqa: E4
 
 SLOTS = {0: "fast loop (hot_load + batches + flush)", 2: "general-path events (pop_min + handle_event)",
          4: "schedulability scan / idle moves", 5: "take_action + end of round", 6: "reward",
-         7: "observation", 8: "fair policy", 11: "  of which hot_load"}
+         7: "observation", 8: "fair policy", 9: "owed graph + reward at the end of the launch",
+         11: "  of which hot_load"}
 
 cfg = {"num_executors": 10, "job_arrival_cap": 50, "job_arrival_rate": 4.0e-5,
        "moving_delay": 2000.0, "warmup_delay": 1000.0}

@@ -109,6 +109,8 @@ k_rollout_fair(Params p, int num_decisions, int dynamic_partition, int auto_rese
 #ifdef SSB_PROFILE
     const long long t_start = clock64();
 #endif
+    // Only the observation that is live when the loop ends is read (by the caller, after the launch): the decisions
+    // write its header and counters, the graph (and the reward, without traj) is left owed and written once at the end.
     int d = 0, fresh = 0;
     while (d < num_decisions) {
         if (sim.h->error) break;
@@ -121,7 +123,7 @@ k_rollout_fair(Params p, int num_decisions, int dynamic_partition, int auto_rese
             const bool was_trunc = !sim.h->done;
             __syncwarp();
             if (lane == 0) { sim.h->reset_count += 1; if (was_trunc) sim.stats->episodes++; }
-            sim.reset_w(seed, tl);
+            sim.reset_w(seed, tl);  // writes its observation in full (or, on a capacity error, a zeroed header): owes nothing
             continue;
         }
         int a = -1, n = 1;
@@ -133,7 +135,7 @@ k_rollout_fair(Params p, int num_decisions, int dynamic_partition, int auto_rese
         if (lane == 0) p.prof[(size_t)b * 16 + 8] += (unsigned long long)(clock64() - tp0);
 #endif
         const double wall0 = sim.oh->wall_time;
-        sim.template step_w<NS>(a, n);
+        sim.template step_w<NS, true>(a, n, 0, traj != nullptr);
         if (traj && lane == 0) {  // RolloutBuffer.add (rollout_worker.py:34-40) minus the observation
             ssb_transition t;
             t.wall_time = wall0; t.reward = sim.oh->reward; t.stage_idx = a; t.num_exec = n;
@@ -144,6 +146,8 @@ k_rollout_fair(Params p, int num_decisions, int dynamic_partition, int auto_rese
         fresh = 0;
         d++;
     }
+    __syncwarp();
+    if (sim.h->obs_owed) sim.finish_obs_w();
 #ifdef SSB_PROFILE
     if (lane == 0) p.prof[(size_t)b * 16 + 10] += (unsigned long long)(clock64() - t_start);
 #endif

@@ -1505,6 +1505,23 @@ struct Sim {
     }
 
     // ------------------------------------------------------------ _observe (:345-406, utils.py:5-22)
+    // edges of a job's template (ne entries from eb) with both ends active: the job's edges in the observation
+    // (utils.subgraph, utils.py:5-22); one thread per job
+    __device__ int job_obs_edges(uint64_t active, int eb, int ne) const
+    {
+        int c = 0;
+#pragma unroll 8
+        for (int k = 0; k < ne; k++) {
+            const int u = p.b_edges[2 * (eb + k)], v = p.b_edges[2 * (eb + k) + 1];
+            c += (int)((active >> u) & (active >> v) & 1);
+        }
+        return c;
+    }
+    // What observe_w writes: OBS_FULL = header, observation counters and the graph slabs (dag_ptr, exec_supplies,
+    // nodes, edge_links).  The fused rollout splits it: OBS_HDR every decision (the header and the counters, from
+    // a count pass with one lane per active job), OBS_GRAPH once when its decision loop ends (the slabs only).
+    enum : int { OBS_HDR = 1, OBS_GRAPH = 2, OBS_FULL = OBS_HDR | OBS_GRAPH };
+    template <int PARTS = OBS_FULL>
     __device__ SSB_COLD void observe_w(double reward, bool terminated)
     {
         const int n_active = h->n_active;
@@ -1513,63 +1530,81 @@ struct Sim {
         int32_t *dag_ptr = p.obs_dag_ptr + (size_t)b * (p.Jc + 1);
         int32_t *sup = p.obs_supplies + (size_t)b * p.Jc;
         const int src_job = source_job_id();
-        int src_idx = n_active, N = 0;
-        // dag_ptr / exec_supplies / source_job_idx: exclusive scan of per-job active-stage counts
-        for (int base = 0; base < n_active; base += 32) {
-            int i = base + lane, cnt = 0, j = -1;
-            if (i < n_active) {
-                j = act[i];
-                cnt = popc64(jb[j].active);
-                sup[i] = jb[j].supply;
+        int src_idx = n_active, N = 0, M = 0;
+        if constexpr (PARTS == OBS_HDR) {
+            for (int base = 0; base < n_active; base += 32) {
+                const int i = base + lane;
+                int j = -1;
+                if (i < n_active) {
+                    j = act[i];
+                    const JobRec &J = jb[j];
+                    const uint64_t active = J.active;
+                    const int eb = p.b_edge_base[J.tmpl];
+                    N += popc64(active);
+                    M += job_obs_edges(active, eb, p.b_edge_base[J.tmpl + 1] - eb);
+                }
+                unsigned hit = __ballot_sync(FULL, j >= 0 && j == src_job);
+                if (hit) src_idx = base + __ffs(hit) - 1;
             }
-            int incl = cnt;
+            N = __reduce_add_sync(FULL, N);
+            M = __reduce_add_sync(FULL, M);
+        } else {
+            // dag_ptr / exec_supplies / source_job_idx: exclusive scan of per-job active-stage counts
+            for (int base = 0; base < n_active; base += 32) {
+                int i = base + lane, cnt = 0, j = -1;
+                if (i < n_active) {
+                    j = act[i];
+                    cnt = popc64(jb[j].active);
+                    sup[i] = jb[j].supply;
+                }
+                int incl = cnt;
 #pragma unroll
-            for (int off = 1; off < 32; off <<= 1) {
-                int v = __shfl_up_sync(FULL, incl, off);
-                if (lane >= off) incl += v;
+                for (int off = 1; off < 32; off <<= 1) {
+                    int v = __shfl_up_sync(FULL, incl, off);
+                    if (lane >= off) incl += v;
+                }
+                if (i < n_active) dag_ptr[i + 1] = N + incl;
+                unsigned hit = __ballot_sync(FULL, j >= 0 && j == src_job);
+                if (hit) src_idx = base + __ffs(hit) - 1;
+                N += __shfl_sync(FULL, incl, 31);
             }
-            if (i < n_active) dag_ptr[i + 1] = N + incl;
-            unsigned hit = __ballot_sync(FULL, j >= 0 && j == src_job);
-            if (hit) src_idx = base + __ffs(hit) - 1;
-            N += __shfl_sync(FULL, incl, 31);
+            if (lane == 0) dag_ptr[0] = 0;
+            __syncwarp();
+            // nodes and edges, one active job at a time, lanes over its stages / template edges
+            for (int i = 0; i < n_active; i++) {
+                const int j = act[i];
+                const JobRec &J = jb[j];
+                const uint64_t active = J.active, sched = J.sched;
+                const int nbase = dag_ptr[i], ns = J.n_stages;
+                for (int s = lane; s < ns; s += 32) {
+                    if (active & bit64(s)) {
+                        const StageRec r = st[J.node_base + s];
+                        int rank = nbase + popc64(active & (bit64(s) - 1));
+                        nodes[rank * 3 + 0] = (float)r.remaining;
+                        nodes[rank * 3 + 1] = r.mrd;
+                        nodes[rank * 3 + 2] = (sched & bit64(s)) ? 1.0f : 0.0f;
+                    }
+                }
+                const int eb = p.b_edge_base[J.tmpl], ne = p.b_edge_base[J.tmpl + 1] - eb;
+                for (int k0 = 0; k0 < ne; k0 += 32) {
+                    int k = k0 + lane, u = 0, v = 0;
+                    bool keep = false;
+                    if (k < ne) {
+                        u = p.b_edges[2 * (eb + k)];
+                        v = p.b_edges[2 * (eb + k) + 1];
+                        keep = (active & bit64(u)) && (active & bit64(v));
+                    }
+                    unsigned m = __ballot_sync(FULL, keep);
+                    if (keep) {
+                        int pos = M + __popc(m & ((1u << lane) - 1));
+                        edges[2 * pos] = nbase + popc64(active & (bit64(u) - 1));
+                        edges[2 * pos + 1] = nbase + popc64(active & (bit64(v) - 1));
+                    }
+                    M += __popc(m);
+                }
+            }
         }
-        if (lane == 0) dag_ptr[0] = 0;
-        __syncwarp();
-        // nodes and edges, one active job at a time, lanes over its stages / template edges
-        int M = 0;
-        for (int i = 0; i < n_active; i++) {
-            const int j = act[i];
-            const JobRec &J = jb[j];
-            const uint64_t active = J.active, sched = J.sched;
-            const int nbase = dag_ptr[i], ns = J.n_stages;
-            for (int s = lane; s < ns; s += 32) {
-                if (active & bit64(s)) {
-                    const StageRec r = st[J.node_base + s];
-                    int rank = nbase + popc64(active & (bit64(s) - 1));
-                    nodes[rank * 3 + 0] = (float)r.remaining;
-                    nodes[rank * 3 + 1] = r.mrd;
-                    nodes[rank * 3 + 2] = (sched & bit64(s)) ? 1.0f : 0.0f;
-                }
-            }
-            const int eb = p.b_edge_base[J.tmpl], ne = p.b_edge_base[J.tmpl + 1] - eb;
-            for (int k0 = 0; k0 < ne; k0 += 32) {
-                int k = k0 + lane, u = 0, v = 0;
-                bool keep = false;
-                if (k < ne) {
-                    u = p.b_edges[2 * (eb + k)];
-                    v = p.b_edges[2 * (eb + k) + 1];
-                    keep = (active & bit64(u)) && (active & bit64(v));
-                }
-                unsigned m = __ballot_sync(FULL, keep);
-                if (keep) {
-                    int pos = M + __popc(m & ((1u << lane) - 1));
-                    edges[2 * pos] = nbase + popc64(active & (bit64(u) - 1));
-                    edges[2 * pos + 1] = nbase + popc64(active & (bit64(v) - 1));
-                }
-                M += __popc(m);
-            }
-        }
-        if (lane == 0) {
+        if ((PARTS & OBS_HDR) && lane == 0) {
             ssb_obs_hdr o;
             o.reward = reward;
             o.wall_time = h->wall_time;
@@ -1636,6 +1671,11 @@ struct Sim {
     // step_begin_w: _take_action and, when the commitment round is over, its bookkeeping (:190-199).
     // Returns 0 when the step is already complete (same-round observation written, or the action was
     // rejected), 1 when the simulation has to advance.
+    // DEFER (the fused rollout): observations are written as OBS_HDR only, and h->obs_owed is set to the parts of the
+    // live observation that finish_obs_w still has to write (OWE_*); a rejected action leaves it as it is.  (In the
+    // header rather than a register: a register live across the decision loop costs the one-slot kernel spills.)
+    enum : int { OWE_GRAPH = 1, OWE_REWARD = 2 };
+    template <bool DEFER = false>
     __device__ __forceinline__ int step_begin_w(int stage_idx, int num_exec)
     {
         SSB_T0();
@@ -1649,7 +1689,16 @@ struct Sim {
             return 0;
         }
         if (lane == 0) stats->decisions++;
-        if (rc == 0) { SSB_TACC(5); observe_w(0.0, false); SSB_TACC(7); return 0; }
+        if (rc == 0) {
+            SSB_TACC(5);
+            if constexpr (DEFER) {  // reward 0: no time passed
+                observe_w<OBS_HDR>(0.0, false);
+                if (lane == 0) h->obs_owed = OWE_GRAPH;
+            }
+            else observe_w(0.0, false);
+            SSB_TACC(7);
+            return 0;
+        }
         // commitment round has completed (:195-199)
         const int n_active0 = h->n_active;
         for (int i = lane; i < n_active0; i += 32) p.old_act[(size_t)b * p.Jc + i] = act[i];
@@ -1671,10 +1720,13 @@ struct Sim {
         return 1;
     }
     // step_end_w: reward, termination flag and the next observation (:201-221)
-    __device__ __forceinline__ void step_end_w()
+    // (DEFER: the reward only when want_reward, else it is owed)
+    template <bool DEFER = false>
+    __device__ __forceinline__ void step_end_w(bool want_reward = true)
     {
         SSB_T0();
-        double reward = -compute_jobtime_w();
+        double reward = 0.0;
+        if (!DEFER || want_reward) reward = -compute_jobtime_w();
         bool terminated = false;
         if (lane == 0) {
             h->pending = 0;
@@ -1685,16 +1737,22 @@ struct Sim {
         terminated = __shfl_sync(FULL, (int)terminated, 0);
         __syncwarp();
         SSB_TACC(6);
-        observe_w(reward, terminated);
+        if constexpr (DEFER) {
+            observe_w<OBS_HDR>(reward, terminated);
+            if (lane == 0) h->obs_owed = want_reward ? OWE_GRAPH : OWE_GRAPH | OWE_REWARD;
+        } else {
+            observe_w(reward, terminated);
+        }
         SSB_TACC(7);
     }
-    template <int NS = 1>
-    __device__ void step_w(int stage_idx, int num_exec, int max_events = 0)
+    // DEFER: see step_begin_w; only for max_events <= 0 (every call reaches its decision)
+    template <int NS = 1, bool DEFER = false>
+    __device__ void step_w(int stage_idx, int num_exec, int max_events = 0, bool want_reward = true)
     {
         if (h->error >= 1000) { if (lane == 0) oh->error = h->error; __syncwarp(); return; }
         if (h->done) { if (lane == 0) oh->error = SSB_ENV_DONE; __syncwarp(); return; }
         if (!h->pending) {
-            if (step_begin_w(stage_idx, num_exec) == 0) return;
+            if (step_begin_w<DEFER>(stage_idx, num_exec) == 0) return;
         }
         bool reached = true;
         if (!h->error) reached = resume_simulation_w<NS>(max_events);
@@ -1708,7 +1766,23 @@ struct Sim {
             __syncwarp();
             return;
         }
-        step_end_w();
+        step_end_w<DEFER>(want_reward);
+    }
+    // the parts of the live observation a deferred step left owed (step_begin_w), written from the current state:
+    // exact as long as nothing has changed the state since that step (compute_jobtime_w writes only its scratch)
+    __device__ SSB_RARE void finish_obs_w()
+    {
+        SSB_T0();
+        const int owed = h->obs_owed;
+        if (owed & OWE_REWARD) {
+            const double reward = -compute_jobtime_w();
+            if (lane == 0) oh->reward = reward;
+            __syncwarp();
+        }
+        if (owed & OWE_GRAPH) observe_w<OBS_GRAPH>(0.0, false);
+        if (lane == 0) h->obs_owed = 0;
+        __syncwarp();
+        SSB_TACC(9);
     }
 
     // StochasticTimeLimit (wrappers/stochastic_time_limit.py:19-21): the episode's time limit ~ Exp(mean), drawn on
@@ -1784,6 +1858,7 @@ struct Sim {
             H.pending = 0;
             H.policy_draws = 0;
             H.hist_n = 0;
+            H.obs_owed = 0;
         }
         __syncwarp();
         if (h->error) {
@@ -2043,13 +2118,7 @@ struct Sim {
         a.supply = J.supply; a.ns = J.n_stages; a.node_base = J.node_base; a.ts_base = J.ts_base;
         a.eb = p.b_edge_base[J.tmpl];
         a.ne = p.b_edge_base[J.tmpl + 1] - a.eb;
-        int c = 0;
-#pragma unroll 8
-        for (int k = 0; k < a.ne; k++) {
-            const int u = p.b_edges[2 * (a.eb + k)], v = p.b_edges[2 * (a.eb + k) + 1];
-            c += (int)((a.active >> u) & (a.active >> v) & 1);
-        }
-        a.n_edges = c;
+        a.n_edges = job_obs_edges(a.active, a.eb, a.ne);
         return a;
     }
     // the i-th active job's share of decima_obs_w (env_wrapper.py:69-143, decima/utils.py:238-267): node rows N..,

@@ -109,7 +109,8 @@ struct __align__(16) EnvHdr {
     int32_t n_edges_total, reset_count, use_tape, pending;
     uint32_t policy_draws;  // Philox policy-stream counter (on-device action sampling)
     int32_t hist_n;         // add_history calls of this episode (rows beyond hist_cap are counted, not stored)
-    int32_t pad2[2];
+    int32_t obs_owed;  // k_rollout_fair: parts of the live observation still to be written (Sim::OWE_*), 0 outside it
+    int32_t pad2;
 };
 
 // Everything a kernel needs, passed by value.
