@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define SSB_ABI_VERSION 6
+#define SSB_ABI_VERSION 7
 
 /* status codes of the entry points */
 enum {
@@ -300,6 +300,19 @@ int ssb_group_baselines(const ssb_transition *traj, const double *returns, const
 /* evaluates the built-in policy on the current observations -> DEVICE i32[B] each */
 int ssb_fair_actions(ssb_env *env, int32_t dynamic_partition, int32_t *stage_idx, int32_t *num_exec,
                      void *stream);
+
+/* RandomScheduler.schedule (random_scheduler.py:7-32) on the device, one decision per env with mask[i] != 0
+ * (mask NULL = all); DEVICE i32[B] outputs; advances each served env's RANDOM-stream counter.
+ * The law is the reference's: a job drawn uniformly among the active jobs that have a schedulable stage, its
+ * find_stage choice as stage_idx (-1 when there is none), num_exec uniform on [1, num_committable_execs].  The draws
+ * come from the episode seed's Philox RANDOM stream (ctr (decision index in the episode, 0, 5, 0);
+ * tests/random_policy_spec.py), not from the reference's RandomState.  Envs that are done, frozen by an
+ * error, pending or masked out get (-1, 1) and keep their counter. */
+int ssb_random_actions(ssb_env *env, const uint8_t *mask, int32_t *stage_idx, int32_t *num_exec, void *stream);
+/* fused random-policy rollout: ssb_rollout_fair's contract with the random policy; traj (DEVICE
+ * ssb_transition[B][num_decisions], lgprob 0) may be NULL */
+int ssb_rollout_random(ssb_env *env, int32_t num_decisions, int32_t auto_reset, uint64_t seed_step,
+                       ssb_transition *traj, void *stream);
 
 int ssb_get_views(ssb_env *env, ssb_views *out);
 

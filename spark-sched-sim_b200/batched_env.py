@@ -258,6 +258,41 @@ class BatchedSparkSchedSimEnv:
         torch.cuda.current_stream(self.device).synchronize()
         return host[:nbytes].numpy().view(nat.TRANSITION_DTYPE).reshape(self.num_envs, int(num_decisions))
 
+    def random_actions(self, mask=None):
+        """The random scheduler (RandomScheduler, random_scheduler.py:7-32) on the device: one action per env with
+        mask[i] != 0 (None = all), drawn from the env's Philox RANDOM stream (a function of the episode seed and the
+        decision's index in the episode).  Envs that are done, pending or masked out get (-1, 1) and keep their
+        draws.  Returns device int32 tensors (stage_idx, num_exec)."""
+        a = torch.empty(self.num_envs, dtype=torch.int32, device=self.device)
+        n = torch.empty(self.num_envs, dtype=torch.int32, device=self.device)
+        m = self._dev(mask, torch.uint8)
+        self._keep = (m,)
+        nat.check(self.L.ssb_random_actions(self._h, m.data_ptr() if m is not None else None, a.data_ptr(),
+                                            n.data_ptr(), self._stream()), "ssb_random_actions")
+        return a, n
+
+    def rollout_random(self, num_decisions, auto_reset=True, seed_step=1, record=False,
+                       out: "torch.Tensor | None" = None, host: "torch.Tensor | None" = None):
+        """rollout_fair with the random scheduler: `num_decisions` decisions per env in one launch.  With
+        record=True every transition is stored (lgprob 0) and returned as rollout_fair_traj returns it: the uint8
+        device tensor `out` (allocated if None), or with `host` (pinned, same size) the structured numpy array
+        [B, num_decisions] of _native.TRANSITION_DTYPE."""
+        if not record:
+            nat.check(self.L.ssb_rollout_random(self._h, int(num_decisions), int(auto_reset), int(seed_step), None,
+                                                self._stream()), "ssb_rollout_random")
+            return None
+        nbytes = self.num_envs * int(num_decisions) * nat.TRANSITION_DTYPE.itemsize
+        if out is None:
+            out = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        assert out.numel() >= nbytes and out.is_cuda
+        nat.check(self.L.ssb_rollout_random(self._h, int(num_decisions), int(auto_reset), int(seed_step),
+                                            out.data_ptr(), self._stream()), "ssb_rollout_random")
+        if host is None:
+            return out
+        host[:nbytes].copy_(out[:nbytes], non_blocking=True)
+        torch.cuda.current_stream(self.device).synchronize()
+        return host[:nbytes].numpy().view(nat.TRANSITION_DTYPE).reshape(self.num_envs, int(num_decisions))
+
     # ---------------------------------------------------------------- host-buffer API (e2e path)
     def reset_host(self, seeds: np.ndarray, time_limits: np.ndarray | None = None,
                    mask: np.ndarray | None = None, grow: bool = False, grow_limit: int = 1 << 16) -> np.ndarray:

@@ -17,14 +17,6 @@
 #include "ssb_env.cuh"
 #include "ssb_sim.cuh"
 
-#ifndef SSB_NS1_CTAS
-#define SSB_NS1_CTAS 7  // resident CTAs per SM of the one-slot kernels: 4096 envs = 1024 CTAs of 4 warps must all be resident
-#endif
-#ifndef SSB_NS2_CTAS
-#define SSB_NS2_CTAS 7  // resident CTAs per SM the two-slot kernels (E > 32) are compiled for: 72 registers (some spilling), but 28 warps
-                        // per SM and 8192 envs = 2048 CTAs in exactly two rounds of resident CTAs (A/B in profiles/r02_ns2_occupancy.txt)
-#endif
-
 using namespace ssb;
 
 namespace ssb {

@@ -24,6 +24,14 @@ extern thread_local char g_cuda_err[256];  // ssb_last_cuda_error()
 #define SSB_WARPS_PER_CTA 4
 #endif
 constexpr int WARPS_PER_CTA = SSB_WARPS_PER_CTA;
+// resident CTAs per SM that the simulator kernels' __launch_bounds__ ask for (fused rollouts of ssb_api.cu and ssb_random.cu)
+#ifndef SSB_NS1_CTAS
+#define SSB_NS1_CTAS 7  // resident CTAs per SM of the one-slot kernels: 4096 envs = 1024 CTAs of 4 warps must all be resident
+#endif
+#ifndef SSB_NS2_CTAS
+#define SSB_NS2_CTAS 7  // resident CTAs per SM the two-slot kernels (E > 32) are compiled for: 72 registers (some spilling), but 28 warps
+                        // per SM and 8192 envs = 2048 CTAs in exactly two rounds of resident CTAs (A/B in profiles/r02_ns2_occupancy.txt)
+#endif
 
 #define CUDA_TRY(expr)                                                                   \
     do {                                                                                 \

@@ -2098,6 +2098,60 @@ struct Sim {
         num_exec = ncommit;
     }
 
+#ifdef SSB_RANDOM_POLICY
+    // ------------------------------------------------------------ random policy
+    // (compiled only in ssb_random.cu, so that the simulator's translation unit is unchanged)
+    // RandomScheduler.schedule (schedulers/heuristics/random_scheduler.py:7-32) in law: the reference redraws a job
+    // uniformly from the jobs still "running" until find_stage gives a stage, i.e. one uniform draw over the active
+    // jobs that have a schedulable stage ("eligible"); num_exec ~ U[1, num_committable].  Draws: the RANDOM stream,
+    // Philox ctr (policy_draws, 0, 5, 0), key = episode seed (tests/random_policy_spec.py); every call
+    // advances policy_draws, also when no job is eligible (stage_idx = -1).
+    __device__ void random_action_w(int &stage_idx, int &num_exec)
+    {
+        const int Ja = h->n_active, ncommit = num_committable();
+        const uint32_t pd = h->policy_draws;
+        int k = 0;  // eligible jobs
+#pragma unroll 1  // (both loops: unrolled, they cost the one-slot rollout kernel spills)
+        for (int base = 0; base < Ja; base += 32) {
+            const int i = base + lane;
+            k += __popc(__ballot_sync(FULL, i < Ja && jb[act[i]].sched != 0));
+        }
+        const uint4 w = philox4x32_10(pd, 0u, 5u, 0u, (uint32_t)h->seed, (uint32_t)(h->seed >> 32));
+        const int t = (int)bounded(w.x, (uint32_t)k);  // the t-th eligible job in active-job order
+        num_exec = 1 + (int)bounded(w.y, (uint32_t)max(ncommit, 0));
+        stage_idx = -1;
+        int run = 0, seen = 0;  // schedulable stages / eligible jobs before this chunk
+#pragma unroll 1
+        for (int base = 0; base < Ja && k > 0; base += 32) {
+            const int i = base + lane;
+            uint64_t m = 0;
+            int below = 0;  // schedulable stages of this job before its find_stage choice
+            bool el = false;
+            if (i < Ja) {
+                const int j = act[i];
+                m = jb[j].sched;
+                if (m) {  // find_stage: first schedulable frontier stage, else first schedulable
+                    const uint64_t f = m & jb[j].frontier;
+                    below = popc64(m & (bit64(ffs64(f ? f : m)) - 1));
+                    el = true;
+                }
+            }
+            const unsigned eb = __ballot_sync(FULL, el);
+            if (t < seen + __popc(eb)) {
+                const int l = __fns(eb, 0, t - seen + 1);  // lane of the (t - seen)-th eligible job of the chunk
+                run += (int)__reduce_add_sync(FULL, lane < l ? (unsigned)popc64(m) : 0u);
+                stage_idx = run + __shfl_sync(FULL, below, l);
+                break;
+            }
+            seen += __popc(eb);
+            run += (int)__reduce_add_sync(FULL, (unsigned)popc64(m));
+        }
+        __syncwarp();
+        if (lane == 0) h->policy_draws = pd + 1;
+        __syncwarp();
+    }
+#endif
+
 #ifdef SSB_DECIMA_CTA_ADAPTER
     // ------------------------------------------------------------ Decima adapter, one CTA per environment
     // (k_decima_obs_cta, ssb_policy.cu; compiled only there so that the simulator's translation unit is unchanged).
