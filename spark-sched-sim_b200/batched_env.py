@@ -245,13 +245,19 @@ class BatchedSparkSchedSimEnv:
         B * num_decisions * 32 bytes (allocated if None).  With `host` (a pinned uint8 tensor of the same
         size) the records are copied to the host and returned as a structured numpy array
         [B, num_decisions] of _native.TRANSITION_DTYPE; otherwise the device tensor is returned."""
+        return self._recorded(num_decisions, out, host, lambda traj: nat.check(
+            self.L.ssb_rollout_fair_traj(self._h, int(num_decisions), int(dynamic_partition), int(auto_reset),
+                                         int(seed_step), traj, self._stream()), "ssb_rollout_fair_traj"))
+
+    def _recorded(self, num_decisions, out, host, launch):
+        """Runs launch(device pointer) on a trajectory buffer for B * num_decisions transition rows: `out` (a uint8
+        device tensor of at least that size; allocated if None).  Returns `out`, or with `host` (pinned uint8 of the
+        same size) the rows copied to the host as a structured array [B, num_decisions] of _native.TRANSITION_DTYPE."""
         nbytes = self.num_envs * int(num_decisions) * nat.TRANSITION_DTYPE.itemsize
         if out is None:
             out = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
         assert out.numel() >= nbytes and out.is_cuda
-        nat.check(self.L.ssb_rollout_fair_traj(self._h, int(num_decisions), int(dynamic_partition),
-                                               int(auto_reset), int(seed_step), out.data_ptr(),
-                                               self._stream()), "ssb_rollout_fair_traj")
+        launch(out.data_ptr())
         if host is None:
             return out
         host[:nbytes].copy_(out[:nbytes], non_blocking=True)
@@ -281,17 +287,9 @@ class BatchedSparkSchedSimEnv:
             nat.check(self.L.ssb_rollout_random(self._h, int(num_decisions), int(auto_reset), int(seed_step), None,
                                                 self._stream()), "ssb_rollout_random")
             return None
-        nbytes = self.num_envs * int(num_decisions) * nat.TRANSITION_DTYPE.itemsize
-        if out is None:
-            out = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
-        assert out.numel() >= nbytes and out.is_cuda
-        nat.check(self.L.ssb_rollout_random(self._h, int(num_decisions), int(auto_reset), int(seed_step),
-                                            out.data_ptr(), self._stream()), "ssb_rollout_random")
-        if host is None:
-            return out
-        host[:nbytes].copy_(out[:nbytes], non_blocking=True)
-        torch.cuda.current_stream(self.device).synchronize()
-        return host[:nbytes].numpy().view(nat.TRANSITION_DTYPE).reshape(self.num_envs, int(num_decisions))
+        return self._recorded(num_decisions, out, host, lambda traj: nat.check(
+            self.L.ssb_rollout_random(self._h, int(num_decisions), int(auto_reset), int(seed_step), traj,
+                                      self._stream()), "ssb_rollout_random"))
 
     # ---------------------------------------------------------------- host-buffer API (e2e path)
     def reset_host(self, seeds: np.ndarray, time_limits: np.ndarray | None = None,
@@ -631,16 +629,9 @@ class BatchedSparkSchedSimEnv:
         (wall time, action, lgprob, reward, flags) recorded -- the RolloutBuffer of
         trainers/rollout_worker.py:18-46 minus the observations.  Finished envs follow set_autoreset().
         Returns the device tensor, or with `host` (pinned uint8) a structured array [B, num_decisions]."""
-        nbytes = self.num_envs * int(num_decisions) * nat.TRANSITION_DTYPE.itemsize
-        if out is None:
-            out = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
-        nat.check(self.L.ssb_rollout_decima(self._h, int(num_decisions), int(max_events), out.data_ptr(),
-                                            self._stream()), "ssb_rollout_decima")
-        if host is None:
-            return out
-        host[:nbytes].copy_(out[:nbytes], non_blocking=True)
-        torch.cuda.current_stream(self.device).synchronize()
-        return host[:nbytes].numpy().view(nat.TRANSITION_DTYPE).reshape(self.num_envs, int(num_decisions))
+        return self._recorded(num_decisions, out, host, lambda traj: nat.check(
+            self.L.ssb_rollout_decima(self._h, int(num_decisions), int(max_events), traj, self._stream()),
+            "ssb_rollout_decima"))
 
     def rollout_decima_async(self, max_decisions, rollout_duration, seed_step=1):
         """Fixed-duration Decima rollouts spanning resets (RolloutWorkerAsync.collect_rollout, rollout_worker.py:160-206).

@@ -13,7 +13,7 @@ PKG_DIR = osp.dirname(osp.abspath(__file__))
 SRC = [osp.join(PKG_DIR, "csrc", "ssb_api.cu"), osp.join(PKG_DIR, "csrc", "ssb_policy.cu"),
        osp.join(PKG_DIR, "csrc", "ssb_backward.cu"), osp.join(PKG_DIR, "csrc", "ssb_learn.cu"),
        osp.join(PKG_DIR, "csrc", "ssb_random.cu")]
-DEPS = SRC + [osp.join(PKG_DIR, "csrc", f) for f in ("ssb_sim.cuh", "ssb_types.cuh", "ssb_env.cuh", "ssb_decima.cuh", "ssb_decima_tc.cuh", "ssb_decima_fused.cuh", "ssb_learn.cuh", "ssb_backward.cuh")] + [
+DEPS = SRC + [osp.join(PKG_DIR, "csrc", f) for f in ("ssb_sim.cuh", "ssb_rollout.cuh", "ssb_types.cuh", "ssb_env.cuh", "ssb_decima.cuh", "ssb_decima_tc.cuh", "ssb_decima_fused.cuh", "ssb_learn.cuh", "ssb_backward.cuh")] + [
     osp.join(osp.dirname(PKG_DIR), "include", "ssb.h")]
 OUT = osp.join(PKG_DIR, "_lib", "libssb.so")
 NVCC_FLAGS = [

@@ -15,7 +15,7 @@
 #include <new>
 #include <vector>
 #include "ssb_env.cuh"
-#include "ssb_sim.cuh"
+#include "ssb_rollout.cuh"
 
 using namespace ssb;
 
@@ -56,13 +56,7 @@ k_step(Params p, const int32_t *stage_idx, const int32_t *num_exec, const uint8_
         if (lane == 0) { next_a[b] = a; next_n[b] = n; }
     };
     if (auto_reset && !sim.h->error && (sim.h->done || sim.oh->truncated)) {
-        // the caller's `if terminated or truncated: env.reset(seed=...)` (rollout_worker.py:118-120, :150-153)
-        const uint64_t seed = sim.h->base_seed + seed_step * (uint64_t)sim.h->reset_count;
-        const double tl = sim.next_time_limit(seed);
-        const bool was_trunc = !sim.h->done;
-        __syncwarp();
-        if (lane == 0) { sim.h->reset_count += 1; if (was_trunc) sim.stats->episodes++; }
-        sim.reset_w(seed, tl);
+        auto_reset_w(sim, lane, seed_step);
         if (lane == 0) sim.oh->was_reset = 1;
         __syncwarp();
         suggest();
@@ -97,52 +91,9 @@ k_rollout_fair(Params p, int num_decisions, int dynamic_partition, int auto_rese
 {
     const int b = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (b >= p.B) return;
-    Sim sim(p, b, lane);
-#ifdef SSB_PROFILE
-    const long long t_start = clock64();
-#endif
-    // Only the observation that is live when the loop ends is read (by the caller, after the launch): the decisions
-    // write its header and counters, the graph (and the reward, without traj) is left owed and written once at the end.
-    int d = 0, fresh = 0;
-    while (d < num_decisions) {
-        if (sim.h->error) break;
-        if (sim.h->done || sim.oh->truncated) {
-            if (!auto_reset) break;
-            fresh = 4;
-            // rollout_worker.py:118-120: seed = base_seed + seed_step * reset_count
-            const uint64_t seed = sim.h->base_seed + seed_step * (uint64_t)sim.h->reset_count;
-            const double tl = sim.next_time_limit(seed);
-            const bool was_trunc = !sim.h->done;
-            __syncwarp();
-            if (lane == 0) { sim.h->reset_count += 1; if (was_trunc) sim.stats->episodes++; }
-            sim.reset_w(seed, tl);  // writes its observation in full (or, on a capacity error, a zeroed header): owes nothing
-            continue;
-        }
-        int a = -1, n = 1;
-#ifdef SSB_PROFILE
-        long long tp0 = clock64();
-#endif
-        sim.fair_action_w(dynamic_partition != 0, a, n);
-#ifdef SSB_PROFILE
-        if (lane == 0) p.prof[(size_t)b * 16 + 8] += (unsigned long long)(clock64() - tp0);
-#endif
-        const double wall0 = sim.oh->wall_time;
-        sim.template step_w<NS, true>(a, n, 0, traj != nullptr);
-        if (traj && lane == 0) {  // RolloutBuffer.add (rollout_worker.py:34-40) minus the observation
-            ssb_transition t;
-            t.wall_time = wall0; t.reward = sim.oh->reward; t.stage_idx = a; t.num_exec = n;
-            t.flags = (sim.oh->terminated ? 1 : 0) | (sim.oh->truncated ? 2 : 0) | fresh;
-            t.lgprob = 0.0f;
-            traj[(size_t)b * num_decisions + d] = t;
-        }
-        fresh = 0;
-        d++;
-    }
-    __syncwarp();
-    if (sim.h->obs_owed) sim.finish_obs_w();
-#ifdef SSB_PROFILE
-    if (lane == 0) p.prof[(size_t)b * 16 + 10] += (unsigned long long)(clock64() - t_start);
-#endif
+    rollout_w<NS>(
+        p, b, lane, [](Sim &sim, int dyn, int &a, int &n) { sim.fair_action_w(dyn != 0, a, n); }, dynamic_partition,
+        num_decisions, auto_reset, seed_step, traj);
 }
 
 // RolloutWorkerAsync.collect_rollout (trainers/rollout_worker.py:160-206): the rollout ends when the env's accumulated
@@ -162,25 +113,15 @@ k_rollout_fair_async(Params p, int max_decisions, double duration, int dynamic_p
         if (sim.h->error) break;
         if (sim.h->done || sim.oh->truncated) {  // :196-200, applied when the loop comes back around
             fresh = 4;
-            const uint64_t seed = sim.h->base_seed + seed_step * (uint64_t)sim.h->reset_count;
-            const double tl = sim.next_time_limit(seed);
-            const bool was_trunc = !sim.h->done;
-            __syncwarp();
-            if (lane == 0) { sim.h->reset_count += 1; if (was_trunc) sim.stats->episodes++; }
-            sim.reset_w(seed, tl);
+            auto_reset_w(sim, lane, seed_step);
             continue;
         }
         int a = -1, n = 1;
         sim.fair_action_w(dynamic_partition != 0, a, n);
         const double wall0 = sim.oh->wall_time;
         sim.template step_w<NS>(a, n);
-        if (traj && lane == 0) {  // rollout_buffer.add(obs, elapsed_time, action, lgprob, reward) (:191)
-            ssb_transition t;
-            t.wall_time = elapsed; t.reward = sim.oh->reward; t.stage_idx = a; t.num_exec = n;
-            t.flags = (sim.oh->terminated ? 1 : 0) | (sim.oh->truncated ? 2 : 0) | fresh;
-            t.lgprob = 0.0f;
-            traj[(size_t)b * max_decisions + d] = t;
-        }
+        // rollout_buffer.add(obs, elapsed_time, action, lgprob, reward) (:191)
+        if (traj && lane == 0) traj[(size_t)b * max_decisions + d] = transition_row(sim, elapsed, a, n, fresh);
         elapsed += sim.oh->wall_time - wall0;  // the duration of this step (:194)
         fresh = 0;
         d++;

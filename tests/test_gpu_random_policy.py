@@ -1,6 +1,6 @@
 """The random scheduler on the device (ssb_random_actions, ssb_rollout_random) against the CPU oracle driven with the
-same draws (tests/random_policy_spec.py: the RANDOM stream on the oracle's observation), against the eager step path,
-and at full batch size against its law."""
+same draws (tests/random_policy_spec.py: the RANDOM stream on the oracle's observation), and at full batch size
+against its law.  tests/test_gpu_rollout_deferred_obs.py compares ssb_rollout_random with the eager step path."""
 import numpy as np
 import pytest
 from scipy.stats import chisquare
@@ -228,72 +228,6 @@ def test_transitions_across_resets(bank, K):
         assert done == K
         assert np.concatenate(parts, axis=1).tobytes() == tr.tobytes()
         assert split.hdr().tobytes() == hdr.tobytes()
-
-
-def eager(bank, cfg, seeds, K):
-    """K decisions per env of the eager loop {random_actions(mask=live); step(mask=live)} with auto-reset; envs are
-    masked once they have taken their K decisions."""
-    import torch
-
-    env = make_env(bank, cfg, seeds)
-    env.set_autoreset(True, 1)
-    n_dec = np.zeros(len(seeds), np.int64)
-    rows = [[] for _ in seeds]
-    hdr = env.hdr()
-    while (n_dec < K).any():
-        live = torch.as_tensor((n_dec < K).astype(np.uint8))
-        a, n = env.random_actions(live)
-        wall0 = hdr["wall_time"].copy()
-        env.step(a, n, mask=live)
-        hdr = env.hdr()
-        a, n = a.cpu().numpy(), n.cpu().numpy()
-        for b in np.nonzero((n_dec < K) & (hdr["was_reset"] == 0))[0]:
-            assert hdr["error"][b] == 0
-            rows[b].append((wall0[b], hdr["reward"][b], a[b], n[b], int(hdr["terminated"][b])))
-            n_dec[b] += 1
-    return env, rows
-
-
-def assert_same_state(ref, got):
-    h0, h1 = ref.hdr(), got.hdr()
-    assert h0.tobytes() == h1.tobytes(), [f for f in h0.dtype.names if not np.array_equal(h0[f], h1[f])]
-    assert ref.stats_per_env().tobytes() == got.stats_per_env().tobytes()
-    for b in range(len(h0)):
-        o0, o1 = ref.obs(b, h0), got.obs(b, h1)
-        for k in ("nodes", "edge_links", "dag_ptr", "exec_supplies"):
-            assert o0[k].tobytes() == o1[k].tobytes(), (b, k)
-        for x, y in zip(ref.jobs(b), got.jobs(b)):
-            assert np.asarray(x).tobytes() == np.asarray(y).tobytes(), b
-
-
-@pytest.mark.parametrize("traj", [False, True])
-@pytest.mark.parametrize("E", [10, 50])
-def test_deferred_equals_eager(bank, E, traj):
-    """rollout_random without and with a trajectory buffer is bit-identical to the eager loop: every header field,
-    the graph slabs, the per-env counters and the job times; K is chosen so that env 0's last decision ends its first
-    episode."""
-    import torch
-    from spark_sched_sim_b200 import _native as nat
-
-    cfg = cfg_of(E, 8)
-    seeds = 1234 + np.arange(12)
-    _, rows0, _ = oracle_loop(bank, cfg, seeds[0], 10**9, auto_reset=False)
-    K = len(rows0)
-    ref, rows = eager(bank, cfg, seeds, K)
-    got = make_env(bank, cfg, seeds)
-    if traj:
-        host = torch.empty(len(seeds) * K * nat.TRANSITION_DTYPE.itemsize, dtype=torch.uint8).pin_memory()
-        tr = got.rollout_random(K, record=True, host=host)
-        for b, r in enumerate(rows):
-            for d, (w0, rew, a, n, term) in enumerate(r):
-                t = tr[b, d]
-                assert (t["wall_time"], t["stage_idx"], t["num_exec"], t["flags"] & 1) == (w0, a, n, term), (b, d)
-                assert np.float64(t["reward"]).tobytes() == np.float64(rew).tobytes(), (b, d)
-    else:
-        got.rollout_random(K)
-    h = got.hdr()[0]
-    assert h["terminated"] == 1 and h["reward"] != 0.0
-    assert_same_state(ref, got)
 
 
 def test_full_batch_law_and_determinism(bank):
