@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define SSB_ABI_VERSION 7
+#define SSB_ABI_VERSION 8
 
 /* status codes of the entry points */
 enum {
@@ -313,6 +313,11 @@ int ssb_random_actions(ssb_env *env, const uint8_t *mask, int32_t *stage_idx, in
  * ssb_transition[B][num_decisions], lgprob 0) may be NULL */
 int ssb_rollout_random(ssb_env *env, int32_t num_decisions, int32_t auto_reset, uint64_t seed_step,
                        ssb_transition *traj, void *stream);
+/* fixed-duration random-policy rollout: ssb_rollout_fair_async's contract with the random policy; traj (DEVICE
+ * ssb_transition[B][max_decisions], lgprob 0), num_steps and elapsed may be NULL.  A draw depends only on the episode
+ * seed and the decision's index in the episode, so the same seeds give the same actions as ssb_rollout_random. */
+int ssb_rollout_random_async(ssb_env *env, int32_t max_decisions, double rollout_duration, uint64_t seed_step,
+                             ssb_transition *traj, int32_t *num_steps, double *elapsed, void *stream);
 
 int ssb_get_views(ssb_env *env, ssb_views *out);
 

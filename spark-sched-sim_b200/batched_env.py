@@ -222,14 +222,18 @@ class BatchedSparkSchedSimEnv:
     def rollout_fair_async(self, max_decisions, rollout_duration, dynamic_partition=True, seed_step=1):
         """Fixed-duration rollouts spanning resets (RolloutWorkerAsync.collect_rollout, rollout_worker.py:160-206).
         Returns (traj uint8 device tensor [B * max_decisions * 32], num_steps i32[B], elapsed f64[B])."""
+        return self._async(max_decisions, lambda traj, num, el: nat.check(
+            self.L.ssb_rollout_fair_async(self._h, int(max_decisions), float(rollout_duration), int(dynamic_partition),
+                                          int(seed_step), traj, num, el, self._stream()), "ssb_rollout_fair_async"))
+
+    def _async(self, max_decisions, launch):
+        """Runs launch(traj, num_steps, elapsed) on device pointers to new buffers for a fixed-duration rollout: traj
+        for B * max_decisions transition rows, num_steps i32[B] and elapsed f64[B].  Returns the three tensors."""
         nbytes = self.num_envs * int(max_decisions) * nat.TRANSITION_DTYPE.itemsize
         traj = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
         num = torch.zeros(self.num_envs, dtype=torch.int32, device=self.device)
         el = torch.zeros(self.num_envs, dtype=torch.float64, device=self.device)
-        nat.check(self.L.ssb_rollout_fair_async(self._h, int(max_decisions), float(rollout_duration),
-                                                int(dynamic_partition), int(seed_step), traj.data_ptr(),
-                                                num.data_ptr(), el.data_ptr(), self._stream()),
-                  "ssb_rollout_fair_async")
+        launch(traj.data_ptr(), num.data_ptr(), el.data_ptr())
         return traj, num, el
 
     def set_mean_time_limit(self, mean_ms: float) -> None:
@@ -290,6 +294,15 @@ class BatchedSparkSchedSimEnv:
         return self._recorded(num_decisions, out, host, lambda traj: nat.check(
             self.L.ssb_rollout_random(self._h, int(num_decisions), int(auto_reset), int(seed_step), traj,
                                       self._stream()), "ssb_rollout_random"))
+
+    def rollout_random_async(self, max_decisions, rollout_duration, seed_step=1):
+        """rollout_fair_async with the random scheduler: fixed-duration rollouts spanning resets
+        (RolloutWorkerAsync.collect_rollout, rollout_worker.py:160-206), every row with lgprob 0.  The draws are those
+        of rollout_random from the same seeds.  Returns (traj uint8 device tensor [B * max_decisions * 32], num_steps
+        i32[B], elapsed f64[B])."""
+        return self._async(max_decisions, lambda traj, num, el: nat.check(
+            self.L.ssb_rollout_random_async(self._h, int(max_decisions), float(rollout_duration), int(seed_step), traj,
+                                            num, el, self._stream()), "ssb_rollout_random_async"))
 
     # ---------------------------------------------------------------- host-buffer API (e2e path)
     def reset_host(self, seeds: np.ndarray, time_limits: np.ndarray | None = None,

@@ -96,9 +96,8 @@ k_rollout_fair(Params p, int num_decisions, int dynamic_partition, int auto_rese
         num_decisions, auto_reset, seed_step, traj);
 }
 
-// RolloutWorkerAsync.collect_rollout (trainers/rollout_worker.py:160-206): the rollout ends when the env's accumulated
-// simulated time reaches `duration` (or after max_decisions rows), resets do not end it, and the time axis of the
-// stored rows is that accumulated time.  (A kernel of its own, so that the default rollout kernel stays as measured.)
+// the fixed-duration rollout (ssb_rollout.cuh) with the fair / FIFO policy.  (A kernel of its own, so that the
+// default rollout kernel stays as measured.)
 template <int NS>
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32, NS == 1 ? SSB_NS1_CTAS : SSB_NS2_CTAS)
 k_rollout_fair_async(Params p, int max_decisions, double duration, int dynamic_partition, uint64_t seed_step,
@@ -107,29 +106,9 @@ k_rollout_fair_async(Params p, int max_decisions, double duration, int dynamic_p
     const int b = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (b >= p.B) return;
     Sim sim(p, b, lane);
-    int d = 0, fresh = 0;
-    double elapsed = 0.0;
-    while (d < max_decisions && elapsed < duration) {
-        if (sim.h->error) break;
-        if (sim.h->done || sim.oh->truncated) {  // :196-200, applied when the loop comes back around
-            fresh = 4;
-            auto_reset_w(sim, lane, seed_step);
-            continue;
-        }
-        int a = -1, n = 1;
-        sim.fair_action_w(dynamic_partition != 0, a, n);
-        const double wall0 = sim.oh->wall_time;
-        sim.template step_w<NS>(a, n);
-        // rollout_buffer.add(obs, elapsed_time, action, lgprob, reward) (:191)
-        if (traj && lane == 0) traj[(size_t)b * max_decisions + d] = transition_row(sim, elapsed, a, n, fresh);
-        elapsed += sim.oh->wall_time - wall0;  // the duration of this step (:194)
-        fresh = 0;
-        d++;
-    }
-    if (lane == 0) {
-        if (num_steps) num_steps[b] = d;
-        if (elapsed_out) elapsed_out[b] = elapsed;
-    }
+    rollout_async_w<NS>(
+        sim, b, lane, [](Sim &sim, int dyn, int &a, int &n) { sim.fair_action_w(dyn != 0, a, n); }, dynamic_partition,
+        max_decisions, duration, seed_step, traj, num_steps, elapsed_out);
 }
 
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32) k_decima_obs(Params p)

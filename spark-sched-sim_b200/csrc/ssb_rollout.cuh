@@ -1,6 +1,7 @@
-// ssb_rollout.cuh -- the fused heuristic rollout on top of the simulator (ssb_sim.cuh): its decision loop, templated
-// on the policy so that the fair (ssb_api.cu) and random (ssb_random.cu) kernels run the same loop in their own units,
-// and the auto-reset and transition-row steps it shares with k_step and k_rollout_fair_async.
+// ssb_rollout.cuh -- the fused heuristic rollouts on top of the simulator (ssb_sim.cuh): the decision loops of the
+// fixed-count (rollout_w) and fixed-duration (rollout_async_w) rollouts, templated on the policy so that the fair
+// (ssb_api.cu) and random (ssb_random.cu) kernels run the same loops in their own units, and the auto-reset and
+// transition-row steps they share with k_step.
 #pragma once
 #include "ssb_env.cuh"
 #include "ssb_sim.cuh"
@@ -78,6 +79,41 @@ __device__ __forceinline__ void rollout_w(const Params &p, int b, int lane, cons
 #ifdef SSB_PROFILE
     if (lane == 0) p.prof[(size_t)b * 16 + 10] += (unsigned long long)(clock64() - t_start);
 #endif
+}
+
+// RolloutWorkerAsync.collect_rollout (trainers/rollout_worker.py:160-206) for env b with `policy(sim, policy_arg, a, n)`:
+// the rollout ends when the env's accumulated simulated time reaches `duration` (or after max_decisions rows), resets
+// do not end it, and the time axis of the stored rows is that accumulated time.  The step is the eager one (every
+// decision writes its observation in full).  b, lane and policy_arg as in rollout_w, and sim is constructed by the
+// kernel too: constructed here from p, k_rollout_fair_async's code moves (24 instructions fewer in <1>, 24 more in <2>).
+template <int NS, class Policy>
+__device__ __forceinline__ void rollout_async_w(Sim &sim, int b, int lane, const Policy &policy, int policy_arg,
+                                                int max_decisions, double duration, uint64_t seed_step,
+                                                ssb_transition *traj, int32_t *num_steps, double *elapsed_out)
+{
+    int d = 0, fresh = 0;
+    double elapsed = 0.0;
+    while (d < max_decisions && elapsed < duration) {
+        if (sim.h->error) break;
+        if (sim.h->done || sim.oh->truncated) {  // :196-200, applied when the loop comes back around
+            fresh = 4;
+            auto_reset_w(sim, lane, seed_step);
+            continue;
+        }
+        int a = -1, n = 1;
+        policy(sim, policy_arg, a, n);
+        const double wall0 = sim.oh->wall_time;
+        sim.template step_w<NS>(a, n);
+        // rollout_buffer.add(obs, elapsed_time, action, lgprob, reward) (:191)
+        if (traj && lane == 0) traj[(size_t)b * max_decisions + d] = transition_row(sim, elapsed, a, n, fresh);
+        elapsed += sim.oh->wall_time - wall0;  // the duration of this step (:194)
+        fresh = 0;
+        d++;
+    }
+    if (lane == 0) {
+        if (num_steps) num_steps[b] = d;
+        if (elapsed_out) elapsed_out[b] = elapsed;
+    }
 }
 
 }  // namespace ssb
