@@ -376,12 +376,12 @@ def test_head_mlp_backward_matches_torch_autograd(bank):
 
 
 def test_backward_down_to_node_embeddings_matches_torch_autograd(bank):
-    """ssb_decima_backward vs torch autograd through everything above NodeEncoder, per env: node embeddings h (the
-    numpy oracle's, a leaf) -> DagEncoder -> GlobalEncoder -> stage / executor-count heads -> utils.evaluate ->
-    loss = sum_b c1_b lgprob_b + c2_b entropy_b.  Compared: d loss / d h per env and the summed gradients of the four
-    MLPs' 24 tensors, each within 3e-4 of its largest entry (device h vs oracle h differ by ~1e-6; fp32 atomics)."""
-    import decima_policy as oracle_pol
-    from torch.distributions.utils import clamp_probs
+    """ssb_decima_backward vs torch autograd through everything above NodeEncoder, all envs in one batch
+    (oracle/decima_torch.py in float32): node embeddings h (the restatement's own, a leaf) -> DagEncoder ->
+    GlobalEncoder -> stage / executor-count heads -> utils.evaluate -> loss = sum_b c1_b lgprob_b + c2_b entropy_b.
+    Compared: d loss / d h per env and the summed gradients of the four MLPs' 24 tensors, each within 3e-4 of its
+    largest entry (device h vs reference h differ by ~1e-6; fp32 atomics)."""
+    import decima_torch
 
     from spark_sched_sim_b200.batched_env import BatchedSparkSchedSimEnv
 
@@ -394,14 +394,6 @@ def test_backward_down_to_node_embeddings_matches_torch_autograd(bank):
     env.reset_host(np.arange(B, dtype=np.uint64) + 301)
     keys = list(w.keys())
     flat_off = np.concatenate([[0], np.cumsum([w[k].size for k in keys])])
-    wf = {k: v.astype(np.float32) for k, v in w.items()}
-
-    def mlp(x, Ws, act):
-        x = act(x @ Ws[0].T + Ws[1])
-        x = act(x @ Ws[2].T + Ws[3])
-        return x @ Ws[4].T + Ws[5]
-
-    leaky = lambda t: torch.nn.functional.leaky_relu(t, 0.2)
     g = torch.Generator(device="cuda").manual_seed(3)
     for k in range(22):
         a, n = env.decima_policy()
@@ -411,95 +403,36 @@ def test_backward_down_to_node_embeddings_matches_torch_autograd(bank):
             gw = torch.zeros(20802, device="cuda")
             d_h = env.decima_backward(c1, c2, gw, through_node_encoder=False).cpu()
             assert not gw[:flat_off[18]].any()  # NodeEncoder's tensors: not part of this stage
-            Wt = {i: torch.from_numpy(wf[keys[i]]).requires_grad_() for i in range(18, 42)}
             hdr = env.hdr().copy()
-            act = env.pol_action.cpu().numpy()
             env.decima_obs()
-            loss = 0.0
-            leaves = []
+            obs = {key: t.cpu() for key, t in decima_torch.handle_observation(env, hdr).items()}
+            Wt = decima_torch.weights(w, torch.float32)
+            with torch.no_grad():
+                h = decima_torch.encode_nodes(Wt, obs)
+            h.requires_grad_()
+            out = decima_torch.evaluate_actions(Wt, obs, c1.cpu(), c2.cpu(), h=h, num_executors=E)
+            out["loss"].backward()
             for b in range(B):
                 if hdr["terminated"][b]:
-                    leaves.append(None)
                     continue
-                obs, d = env.obs(b, hdr), env.decima_obs_host(b, hdr)
-                x = d["features"].astype(np.float32)
-                dag_ptr = np.asarray(obs["dag_ptr"])
-                h_np, _, _ = oracle_pol.encode(wf, x, np.asarray(obs["edge_links"]).reshape(-1, 2),
-                                               d["edge_bits"].astype(np.uint64), int(d["depth"]), dag_ptr)
-                h = torch.from_numpy(h_np).requires_grad_()
-                leaves.append(h)
-                xt = torch.from_numpy(x)
-                N, Ja = x.shape[0], len(dag_ptr) - 1
-                z = mlp(torch.cat([xt, h], 1), [Wt[i] for i in range(18, 24)], leaky)
-                seg = torch.from_numpy(np.repeat(np.arange(Ja), np.diff(dag_ptr))).long()
-                h_dag = torch.zeros(Ja, 16).index_add(0, seg, z)
-                h_glob = mlp(h_dag, [Wt[i] for i in range(24, 30)], leaky).sum(0)
-                idx = torch.from_numpy(np.flatnonzero(d["stage_mask"])).long()
-                inp = torch.cat([xt[idx], h[idx], h_dag[seg[idx]], h_glob.expand(len(idx), 16)], 1)
-                zs = mlp(inp, [Wt[i] for i in range(30, 36)], torch.tanh)[:, 0]
-                job, cap = int(act[b, 1]), int(d["commit_caps"][act[b, 1]])
-                cnt = (torch.arange(cap, dtype=torch.float64) / E).float()[:, None]
-                inp = torch.cat([xt[dag_ptr[job], :3].expand(cap, 3), h_dag[job].expand(cap, 16),
-                                 h_glob.expand(cap, 16), cnt], 1)
-                ze = mlp(inp, [Wt[i] for i in range(36, 42)], torch.tanh)[:, 0]
-                lg = en = 0.0
-                for zz, sel in ((zs, int(act[b, 0])), (ze, int(act[b, 2]))):
-                    q = clamp_probs(torch.softmax(zz, 0))
-                    lg = lg + q.log()[sel]
-                    en = en - (q.log() * q).sum()
-                en = en / np.log(np.float32(E * N))
-                loss = loss + float(c1[b]) * lg + float(c2[b]) * en
-            loss.backward()
-            for b in range(B):
-                if leaves[b] is None:
-                    continue
-                N = leaves[b].shape[0]
-                tol = 3e-4 * float(leaves[b].grad.abs().max()) + 3e-6
-                assert float((d_h[b, :N] - leaves[b].grad).abs().max()) <= tol, (k, b)
+                N = int(hdr["num_nodes"][b])
+                tol = 3e-4 * float(h.grad[b].abs().max()) + 3e-6
+                assert float((d_h[b, :N] - h.grad[b, :N]).abs().max()) <= tol, (k, b)
                 assert not d_h[b, N:].any()
             for i in range(18, 42):
-                got = gw[flat_off[i]:flat_off[i + 1]].view(Wt[i].shape).cpu()
-                tol = 3e-4 * float(Wt[i].grad.abs().max()) + 3e-6  # (a last-layer bias gradient is a sum that cancels to ~0: pure rounding)
-                assert float((got - Wt[i].grad).abs().max()) <= tol, (k, keys[i])
+                want = Wt[keys[i]].grad
+                got = gw[flat_off[i]:flat_off[i + 1]].view(want.shape).cpu()
+                tol = 3e-4 * float(want.abs().max()) + 3e-6  # (a last-layer bias gradient is a sum that cancels to ~0: pure rounding)
+                assert float((got - want).abs().max()) <= tol, (k, keys[i])
         env.step(a, n)
-
-
-def _torch_encode(Wt, keys, x, edge_links, edge_bits, depth):
-    """oracle/decima_policy.encode's NodeEncoder (scheduler.py:191-241, overwrite semantics) in torch, functional so
-    that autograd sees every level."""
-    leaky = lambda t: torch.nn.functional.leaky_relu(t, 0.2)
-
-    def mlp(t, first):
-        t = leaky(t @ Wt[first].T + Wt[first + 1])
-        t = leaky(t @ Wt[first + 2].T + Wt[first + 3])
-        return t @ Wt[first + 4].T + Wt[first + 5]
-
-    idx = {k: i for i, k in enumerate(keys)}
-    prep, msg_w, upd = (idx[f"encoder.node_encoder.{n}.0.weight"] for n in ("mlp_prep", "mlp_msg", "mlp_update"))
-    N = x.shape[0]
-    h_init = mlp(x, prep)
-    if depth == 0:
-        return h_init
-    u, v = edge_links[:, 0], edge_links[:, 1]
-    is_src = np.zeros(N, bool); is_src[u] = True
-    sinks = torch.from_numpy(~is_src)
-    h = torch.where(sinks[:, None], mlp(h_init, upd), torch.zeros_like(h_init))
-    for k in reversed(range(depth)):
-        m = ((edge_bits >> np.uint64(k)) & np.uint64(1)).astype(bool)
-        uk, vk = torch.from_numpy(u[m]).long(), torch.from_numpy(v[m]).long()
-        recv = np.zeros(N, bool); recv[u[m]] = True
-        msg = mlp(h, msg_w)  # only the masked children's rows are used
-        agg = torch.zeros_like(h).index_add(0, uk, msg[vk])
-        h = torch.where(torch.from_numpy(recv)[:, None], h_init + mlp(agg, upd), h)
-    return h
 
 
 def test_full_backward_matches_torch_autograd(bank):
     """ssb_decima_backward(through_node_encoder=True): the gradients of all 42 tensors of the shipped model for
-    loss = sum_b c1_b lgprob_b + c2_b entropy_b, against torch autograd through a torch restatement of the whole
-    policy (NodeEncoder with its level loop, DagEncoder, GlobalEncoder, both heads, utils.evaluate) per env.
-    Every tensor within 5e-4 of its largest entry (fp32 atomics; tf32x3 forward vs fp32)."""
-    from torch.distributions.utils import clamp_probs
+    loss = sum_b c1_b lgprob_b + c2_b entropy_b, against torch autograd through oracle/decima_torch.py (the whole
+    policy over all envs in one batch: NodeEncoder with its level loop, DagEncoder, GlobalEncoder, both heads,
+    utils.evaluate) in float32.  Every tensor within 5e-4 of its largest entry (fp32 atomics; tf32x3 forward vs fp32)."""
+    import decima_torch
 
     from spark_sched_sim_b200.batched_env import BatchedSparkSchedSimEnv
 
@@ -512,13 +445,6 @@ def test_full_backward_matches_torch_autograd(bank):
     env.reset_host(np.arange(B, dtype=np.uint64) + 501)
     keys = list(w.keys())
     flat_off = np.concatenate([[0], np.cumsum([w[k].size for k in keys])])
-    leaky = lambda t: torch.nn.functional.leaky_relu(t, 0.2)
-
-    def mlp(x, Ws, act):
-        x = act(x @ Ws[0].T + Ws[1])
-        x = act(x @ Ws[2].T + Ws[3])
-        return x @ Ws[4].T + Ws[5]
-
     g = torch.Generator(device="cuda").manual_seed(9)
     for k in range(22):
         a, n = env.decima_policy()
@@ -526,50 +452,19 @@ def test_full_backward_matches_torch_autograd(bank):
             c1 = torch.randn(B, device="cuda", generator=g)
             c2 = torch.randn(B, device="cuda", generator=g)
             hdr = env.hdr().copy()
-            act = env.pol_action.cpu().numpy()
             env.decima_obs()
-            obs_l = [(env.obs(b, hdr), env.decima_obs_host(b, hdr)) for b in range(B)]
+            obs = {key: t.cpu().clone() for key, t in decima_torch.handle_observation(env, hdr).items()}
             gw = torch.zeros(20802, device="cuda")
             env.decima_backward(c1, c2, gw)
-            Wt = {i: torch.from_numpy(w[keys[i]].astype(np.float32)).requires_grad_() for i in range(42)}
-            loss = 0.0
-            depths = []
-            for b in range(B):
-                if hdr["terminated"][b]:
-                    continue
-                obs, d = obs_l[b]
-                x = torch.from_numpy(d["features"].astype(np.float32))
-                dag_ptr = np.asarray(obs["dag_ptr"])
-                depths.append(int(d["depth"]))
-                h = _torch_encode(Wt, keys, x, np.asarray(obs["edge_links"]).reshape(-1, 2),
-                                  d["edge_bits"].astype(np.uint64), int(d["depth"]))
-                N, Ja = x.shape[0], len(dag_ptr) - 1
-                z = mlp(torch.cat([x, h], 1), [Wt[i] for i in range(18, 24)], leaky)
-                seg = torch.from_numpy(np.repeat(np.arange(Ja), np.diff(dag_ptr))).long()
-                h_dag = torch.zeros(Ja, 16).index_add(0, seg, z)
-                h_glob = mlp(h_dag, [Wt[i] for i in range(24, 30)], leaky).sum(0)
-                idx = torch.from_numpy(np.flatnonzero(d["stage_mask"])).long()
-                inp = torch.cat([x[idx], h[idx], h_dag[seg[idx]], h_glob.expand(len(idx), 16)], 1)
-                zs = mlp(inp, [Wt[i] for i in range(30, 36)], torch.tanh)[:, 0]
-                job, cap = int(act[b, 1]), int(d["commit_caps"][act[b, 1]])
-                cnt = (torch.arange(cap, dtype=torch.float64) / E).float()[:, None]
-                inp = torch.cat([x[dag_ptr[job], :3].expand(cap, 3), h_dag[job].expand(cap, 16),
-                                 h_glob.expand(cap, 16), cnt], 1)
-                ze = mlp(inp, [Wt[i] for i in range(36, 42)], torch.tanh)[:, 0]
-                lg = en = 0.0
-                for zz, sel in ((zs, int(act[b, 0])), (ze, int(act[b, 2]))):
-                    q = clamp_probs(torch.softmax(zz, 0))
-                    lg = lg + q.log()[sel]
-                    en = en - (q.log() * q).sum()
-                en = en / np.log(np.float32(E * N))
-                loss = loss + float(c1[b]) * lg + float(c2[b]) * en
-            loss.backward()
+            Wt = decima_torch.weights(w, torch.float32)
+            decima_torch.evaluate_actions(Wt, obs, c1.cpu(), c2.cpu(), num_executors=E)["loss"].backward()
             if k == 21:
-                assert max(depths) >= 2  # the level loop was exercised
+                assert int(obs["depth"][obs["live"]].max()) >= 2  # the level loop was exercised
             for i in range(42):
-                got = gw[flat_off[i]:flat_off[i + 1]].view(Wt[i].shape).cpu()
-                tol = 5e-4 * float(Wt[i].grad.abs().max()) + 3e-6
-                assert float((got - Wt[i].grad).abs().max()) <= tol, (k, keys[i], float((got - Wt[i].grad).abs().max()), tol)
+                want = Wt[keys[i]].grad
+                got = gw[flat_off[i]:flat_off[i + 1]].view(want.shape).cpu()
+                tol = 5e-4 * float(want.abs().max()) + 3e-6
+                assert float((got - want).abs().max()) <= tol, (k, keys[i], float((got - want).abs().max()), tol)
             # the backward pass overwrote the intermediate buffers: the next policy call recomputes everything
         env.step(a, n)
 
