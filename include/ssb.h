@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define SSB_ABI_VERSION 8
+#define SSB_ABI_VERSION 9
 
 /* status codes of the entry points */
 enum {
@@ -344,7 +344,8 @@ int ssb_get_decima_views(ssb_env *env, ssb_decima_views *out);
  *   weights: HOST, 20 802 floats, the tensors of models/decima/model.pt concatenated in
  *            state_dict order (each row-major).
  *   forced_stage / forced_num_exec: DEVICE i32[B] or NULL; an entry >= 0 replaces the sampled index
- *            (replaying recorded actions); sampling uses the Philox policy stream of the env's seed.
+ *            (replaying recorded actions); sampling uses the Philox DECIMA stream of the env's seed,
+ *            ctr (decision index in the episode, policy stream of the env, 4, 0) (ssb_set_policy_streams).
  *   stage_idx_out / num_exec_out: DEVICE i32[B] or NULL, in the ENV's action format
  *            (DecimaActWrapper, env_wrapper.py:33-34: num_exec + 1), ready for ssb_step. */
 typedef struct {
@@ -360,6 +361,14 @@ int ssb_set_decima_weights(ssb_env *env, const float *weights, int32_t n_floats)
 int ssb_decima_policy(ssb_env *env, const int32_t *forced_stage, const int32_t *forced_num_exec,
                       int32_t *stage_idx_out, int32_t *num_exec_out, void *stream);
 int ssb_get_policy_views(ssb_env *env, ssb_policy_views *out);
+/* Per-env policy sampling streams (the reference's rollout workers each own a torch RNG): streams = HOST u32[B],
+ * NULL = all 0.  Env b's Decima actions are drawn at Philox ctr (decision index in the episode, streams[b], 4, 0),
+ * key = the episode seed, so envs that share a seed (one job sequence, several rollouts) still sample their own
+ * actions; stream 0 is the default and gives the draws of a handle that never called this.  The streams belong to
+ * the handle, not to the episode: ssb_reset, ssb_reset_host, auto-resets and the resets inside the Decima rollouts
+ * keep them.  The random scheduler's RANDOM stream (ssb_random_actions) does not use them.  Synchronises the
+ * device. */
+int ssb_set_policy_streams(ssb_env *env, const uint32_t *streams);
 /* One of the policy's seven MLPs (make_mlp, schedulers/decima/utils.py:45-64) applied to caller-provided rows on the
  * tensor-core path the policy uses: mlp = 0 mlp_prep (5 -> 16), 1 mlp_msg, 2 mlp_update (16 -> 16), 3 DagEncoder
  * (21 -> 16), 4 GlobalEncoder (16 -> 16), 5 stage score head (53 -> 1), 6 executor-count score head (36 -> 1), in
@@ -458,6 +467,17 @@ int ssb_rollout_decima(ssb_env *env, int32_t num_decisions, int32_t max_events, 
  * untouched) and continue where they stopped at the next call.  Synchronises the stream every few rounds. */
 int ssb_rollout_decima_async(ssb_env *env, int32_t max_decisions, double rollout_duration, uint64_t seed_step,
                              ssb_transition *traj, int32_t *num_steps, double *elapsed, void *stream);
+/* The stored observations of the two Decima rollouts (RolloutBuffer.obsns, rollout_worker.py:18-46): while a store
+ * is attached, every transition row (b, d) that ssb_rollout_decima (d = decision index of the call) or
+ * ssb_rollout_decima_async (d = env b's row) writes also stores env b's observation -- the one its action was sampled
+ * on -- in slot b of block d of `snapshots` (DEVICE: capacity consecutive blocks in the ssb_decima_snapshot format,
+ * ssb_decima_snapshot_bytes each; ssb_decima_snapshot_gather reads them), and the Decima-format action at
+ * stage_sel[d][b] / exec_sel[d][b] (DEVICE i32[capacity][B]).  Rows without a transition (re-seed only, a finished
+ * env idling, an env past its duration) write nothing; only the rows in use of each part are written.  The rollouts
+ * refuse (SSB_E_INVALID) num_decisions / max_decisions > capacity.  snapshots == NULL detaches.  Refused while a
+ * snapshot is loaded (ssb_decima_snapshot_load) and on a handle without the policy. */
+int ssb_decima_attach_rollout_store(ssb_env *env, void *snapshots, int32_t capacity, int32_t *stage_sel,
+                                    int32_t *exec_sel);
 /* collect_stats (trainers/rollout_worker.py:122-129) over all envs as SUMS that can be all-reduced across GPUs:
  * out = DEVICE f64[8]: [0] sum over envs of avg_num_jobs = (total job time so far) / wall_time
  * (metrics.py:15-16; envs at wall_time 0 skipped), [1] number of envs counted in [0], [2] completed jobs,

@@ -9,7 +9,7 @@ import numpy as np
 
 PKG_DIR = osp.dirname(osp.abspath(__file__))
 LIB_PATH = osp.join(PKG_DIR, "_lib", "libssb.so")
-ABI_VERSION = 8
+ABI_VERSION = 9
 
 
 class SsbConfig(C.Structure):
@@ -142,7 +142,7 @@ EXPORTS = [
     "ssb_load_trace", "ssb_clear_trace", "ssb_reset", "ssb_step", "ssb_reset_host", "ssb_step_host", "ssb_step_fair_host", "ssb_set_autoreset", "ssb_set_mean_time_limit",
     "ssb_rollout_fair", "ssb_rollout_fair_traj", "ssb_rollout_fair_async", "ssb_discounted_returns", "ssb_differential_returns", "ssb_group_baselines", "ssb_ppo_loss", "ssb_adam_step", "ssb_fair_actions", "ssb_random_actions", "ssb_rollout_random", "ssb_rollout_random_async", "ssb_get_views", "ssb_get_stats", "ssb_collect_stats", "ssb_reset_stats",
     "ssb_get_jobs", "ssb_get_log", "ssb_get_history", "ssb_decima_obs", "ssb_get_decima_views",
-    "ssb_set_decima_weights", "ssb_decima_policy", "ssb_rollout_decima", "ssb_rollout_decima_async", "ssb_decima_snapshot_bytes",
+    "ssb_set_decima_weights", "ssb_decima_policy", "ssb_rollout_decima", "ssb_rollout_decima_async", "ssb_set_policy_streams", "ssb_decima_attach_rollout_store", "ssb_decima_snapshot_bytes",
     "ssb_decima_snapshot", "ssb_decima_snapshot_gather", "ssb_decima_snapshot_load", "ssb_decima_snapshot_unload", "ssb_decima_evaluate", "ssb_decima_head_adjoint", "ssb_decima_head_backward", "ssb_decima_backward_bytes", "ssb_decima_attach_backward_scratch", "ssb_decima_backward", "ssb_get_policy_views", "ssb_decima_work", "ssb_decima_mlp_rows", "ssb_packed_obs_bytes", "ssb_get_obs_host", "ssb_get_debug_counters",
 ]
 
@@ -181,6 +181,8 @@ def lib():
     L.ssb_step_fair_host.argtypes = [vp, vp, vp, vp, i32, i32, vp, vp, vp]
     L.ssb_rollout_decima.argtypes = [vp, i32, i32, vp, vp]
     L.ssb_rollout_decima_async.argtypes = [vp, i32, C.c_double, u64, vp, vp, vp, vp]
+    L.ssb_set_policy_streams.argtypes = [vp, vp]
+    L.ssb_decima_attach_rollout_store.argtypes = [vp, vp, i32, vp, vp]
     L.ssb_decima_snapshot_bytes.argtypes = [vp, C.POINTER(C.c_size_t)]
     L.ssb_decima_snapshot.argtypes = [vp, vp, vp]
     L.ssb_decima_snapshot_gather.argtypes = [vp, vp, i32, vp, vp, vp, vp]

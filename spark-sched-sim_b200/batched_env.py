@@ -134,8 +134,8 @@ class BatchedSparkSchedSimEnv:
     def grow(self, max_jobs: int) -> None:
         """Re-creates the handle with room for `max_jobs` jobs per env (node / edge / pool capacities follow).  The
         capacity is fixed at creation (one workspace, carved once), so growing means a new handle: every env's
-        state is lost (reset afterwards); the policy weights, the auto-reset mode and the mean time limit are
-        carried over.  Time-limited arrivals without a job cap are the case that needs this: an episode that draws
+        state is lost (reset afterwards); the policy weights, the policy sampling streams, the auto-reset mode and the
+        mean time limit are carried over.  Time-limited arrivals without a job cap are the case that needs this: an episode that draws
         more jobs than the capacity stops at its reset with SSB_ENV_CAPACITY (`reset_host(..., grow=True)` grows
         and retries; `required_job_capacity` sizes the handle up front)."""
         assert max_jobs > self.max_jobs
@@ -148,6 +148,8 @@ class BatchedSparkSchedSimEnv:
             self.set_autoreset(*self._settings["autoreset"])
         if "mean_time_limit" in self._settings:
             self.set_mean_time_limit(self._settings["mean_time_limit"])
+        if "policy_streams" in self._settings:
+            self.set_policy_streams(self._settings["policy_streams"])
 
     @staticmethod
     def required_job_capacity(job_arrival_rate: float, mean_time_limit: float, tail: float = 1e-9) -> int:
@@ -482,6 +484,32 @@ class BatchedSparkSchedSimEnv:
                   "ssb_set_decima_weights")
         self._weights = flat
 
+    def set_policy_streams(self, streams) -> None:
+        """Each env's Decima sampling stream (uint32 per env, None = all 0): the actions are drawn at Philox counter
+        (decision index in the episode, stream, 4, 0) keyed by the episode seed, so envs that share a job sequence
+        (same seed) but not a stream sample their own actions, as the reference's rollout workers do with their own
+        torch RNGs.  Stream 0 is the default.  Resets keep the streams."""
+        st = None if streams is None else np.ascontiguousarray(np.asarray(streams, dtype=np.uint32))
+        assert st is None or st.size == self.num_envs
+        nat.check(self.L.ssb_set_policy_streams(self._h, st.ctypes.data if st is not None else None),
+                  "ssb_set_policy_streams")
+        self._settings["policy_streams"] = st
+
+    def _with_store(self, store, run):
+        """run() with `store` (a ppo.RolloutStore of this handle) attached to the handle: the Decima rollouts then also
+        write every transition row's observation and Decima-format action into it.  Detached again afterwards."""
+        if store is None:
+            return run()
+        assert store.env is self and store.snapshots.shape[1] == self.decima_snapshot_bytes()
+        nat.check(self.L.ssb_decima_attach_rollout_store(self._h, store.snapshots.data_ptr(), store.K,
+                                                         store.stage_sel.data_ptr(), store.exec_sel.data_ptr()),
+                  "ssb_decima_attach_rollout_store")
+        try:
+            return run()
+        finally:
+            nat.check(self.L.ssb_decima_attach_rollout_store(self._h, None, 0, None, None),
+                      "ssb_decima_attach_rollout_store")
+
     def decima_policy(self, forced_stage=None, forced_num_exec=None):
         """One Decima decision per env on the device (observation adapter + GNN + sampling).
         Returns (stage_idx, num_exec) device tensors in the env's action format; the scores, the
@@ -637,25 +665,28 @@ class BatchedSparkSchedSimEnv:
         return d_h
 
     def rollout_decima(self, num_decisions, max_events=0, out: "torch.Tensor | None" = None,
-                       host: "torch.Tensor | None" = None):
+                       host: "torch.Tensor | None" = None, store=None):
         """Decima rollout collection on the device: num_decisions x { decima_policy ; step } with every call's
         (wall time, action, lgprob, reward, flags) recorded -- the RolloutBuffer of
-        trainers/rollout_worker.py:18-46 minus the observations.  Finished envs follow set_autoreset().
+        trainers/rollout_worker.py:18-46; with `store` (a ppo.RolloutStore of this handle with room for num_decisions)
+        also the observations and Decima-format actions, row d in its block d.  Finished envs follow set_autoreset().
         Returns the device tensor, or with `host` (pinned uint8) a structured array [B, num_decisions]."""
-        return self._recorded(num_decisions, out, host, lambda traj: nat.check(
+        return self._with_store(store, lambda: self._recorded(num_decisions, out, host, lambda traj: nat.check(
             self.L.ssb_rollout_decima(self._h, int(num_decisions), int(max_events), traj, self._stream()),
-            "ssb_rollout_decima"))
+            "ssb_rollout_decima")))
 
-    def rollout_decima_async(self, max_decisions, rollout_duration, seed_step=1):
+    def rollout_decima_async(self, max_decisions, rollout_duration, seed_step=1, store=None):
         """Fixed-duration Decima rollouts spanning resets (RolloutWorkerAsync.collect_rollout, rollout_worker.py:160-206).
+        With `store` (a ppo.RolloutStore of this handle with room for max_decisions) env b's row d also stores its
+        observation and Decima-format action in the store's block d.
         Returns (traj uint8 device tensor [B * max_decisions * 32], num_steps i32[B], elapsed f64[B])."""
         nbytes = self.num_envs * int(max_decisions) * nat.TRANSITION_DTYPE.itemsize
         traj = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
         num = torch.zeros(self.num_envs, dtype=torch.int32, device=self.device)
         el = torch.zeros(self.num_envs, dtype=torch.float64, device=self.device)
-        nat.check(self.L.ssb_rollout_decima_async(self._h, int(max_decisions), float(rollout_duration), int(seed_step),
-                                                  traj.data_ptr(), num.data_ptr(), el.data_ptr(), self._stream()),
-                  "ssb_rollout_decima_async")
+        self._with_store(store, lambda: nat.check(self.L.ssb_rollout_decima_async(
+            self._h, int(max_decisions), float(rollout_duration), int(seed_step), traj.data_ptr(), num.data_ptr(),
+            el.data_ptr(), self._stream()), "ssb_rollout_decima_async"))
         return traj, num, el
 
     def load_trace(self, b, t_arrival, template, tape=None):

@@ -248,7 +248,7 @@ int compute_dims(const ssb_config &c, const ssb_bank &bk, Dims &d)
 }
 
 void carve(Carver &cv, const ssb_config &c, const ssb_bank &bk, const Dims &d, Params &p, BankDev &bd,
-           int32_t **st_a, int32_t **st_n, uint64_t **st_seed, double **st_tl, uint8_t **st_mask)
+           int32_t **st_a, int32_t **st_n, uint64_t **st_seed, double **st_tl, uint8_t **st_mask, uint32_t **pol_streams)
 {
     const size_t B = c.num_envs, T = bk.num_templates, TS = bk.num_template_stages;
     bd.num_stages = cv.take<int32_t>(T);
@@ -296,7 +296,7 @@ void carve(Carver &cv, const ssb_config &c, const ssb_bank &bk, const Dims &d, P
         p.dec_edge_bits = cv.take<uint64_t>(B * d.Mc);
         p.dec_depth = cv.take<int32_t>(B);
     }
-    if (c.flags & SSB_FLAG_DECIMA_POLICY) ssb_i_policy_carve(cv, c, d, p);
+    if (c.flags & SSB_FLAG_DECIMA_POLICY) ssb_i_policy_carve(cv, c, d, p, pol_streams);
     *st_a = cv.take<int32_t>(B);
     *st_n = cv.take<int32_t>(B);
     *st_seed = cv.take<uint64_t>(B);
@@ -330,8 +330,8 @@ int ssb_workspace_bytes(const ssb_config *cfg, const ssb_bank *bank, size_t *byt
     Carver cv{nullptr};
     Params p{};
     BankDev bd{};
-    int32_t *a, *n; uint64_t *s; double *tl; uint8_t *m;
-    carve(cv, *cfg, *bank, d, p, bd, &a, &n, &s, &tl, &m);
+    int32_t *a, *n; uint64_t *s; double *tl; uint8_t *m; uint32_t *ps;
+    carve(cv, *cfg, *bank, d, p, bd, &a, &n, &s, &tl, &m, &ps);
     *bytes = (cv.off + 255) & ~size_t(255);
     return SSB_OK;
 }
@@ -358,7 +358,8 @@ int ssb_create(const ssb_config *cfg, const ssb_bank *bk, int device, void *work
     Carver cv{env->ws};
     Params &p = env->p;
     p = Params{};
-    carve(cv, *cfg, *bk, d, p, env->bank, &env->st_a, &env->st_n, &env->st_seed, &env->st_tl, &env->st_mask);
+    carve(cv, *cfg, *bk, d, p, env->bank, &env->st_a, &env->st_n, &env->st_seed, &env->st_tl, &env->st_mask,
+          &env->pol_streams);
     p.B = cfg->num_envs; p.E = cfg->num_executors; p.Jc = cfg->max_jobs; p.Sc = d.Sc; p.Mc = d.Mc;
     p.TAB = d.TAB; p.RT = d.RT; p.P = d.P; p.Cc = d.Cc; p.max_stages = d.max_stages;
     p.tape_cap = cfg->tape_capacity; p.log_cap = cfg->log_capacity;

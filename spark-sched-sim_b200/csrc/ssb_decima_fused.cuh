@@ -452,6 +452,7 @@ struct Args {
     int32_t *stage_idx_out, *num_exec_out;          // DEVICE i32[B] or nullptr (env-format action)
     int32_t *cursor;                                // DEVICE, zeroed before the launch: next group
     int run_adapter, advance_draws, group;          // group = environments per group (<= GMAX)
+    const uint32_t *streams;                        // DEVICE u32[B]: each env's policy sampling stream
 };
 
 struct EnvInfo { int b, N, M, Ja, depth, node0, job0, ncand, cap, job_idx; };
@@ -783,7 +784,7 @@ __global__ void __launch_bounds__(THREADS, 2) k_decima_fused(Params p, Args a)
         for (int i = warp; i < ne; i += WARPS) {
             const int b = info[i].b, N = info[i].N, Ja = info[i].Ja, n_cand = info[i].ncand;
             const EnvHdr &h = p.hdr[b];
-            const uint4 rw = philox4x32_10(h.policy_draws, 0u, 4u, 0u, (uint32_t)h.seed, (uint32_t)(h.seed >> 32));
+            const uint4 rw = philox4x32_10(h.policy_draws, a.streams[b], 4u, 0u, (uint32_t)h.seed, (uint32_t)(h.seed >> 32));
             const float u1 = ((float)(rw.x >> 8) + 0.5f) * (1.0f / 16777216.0f);
             float lgprob = 0.0f, h_stage = 0.0f;
             const int stage_idx = n_cand > 0 ? sample_w(p.pol_stage_logits + (size_t)b * p.Sc, n_cand,
@@ -825,7 +826,7 @@ __global__ void __launch_bounds__(THREADS, 2) k_decima_fused(Params p, Args a)
             const int b = info[i].b, cap = info[i].cap;
             EnvHdr &h = p.hdr[b];
             const uint32_t pd = h.policy_draws;
-            const uint4 rw = philox4x32_10(pd, 0u, 4u, 0u, (uint32_t)h.seed, (uint32_t)(h.seed >> 32));
+            const uint4 rw = philox4x32_10(pd, a.streams[b], 4u, 0u, (uint32_t)h.seed, (uint32_t)(h.seed >> 32));
             const float u2 = ((float)(rw.y >> 8) + 0.5f) * (1.0f / 16777216.0f);
             float lgprob = p.pol_lgprob[b], h_exec = 0.0f;
             int num_exec = 0;

@@ -673,7 +673,9 @@ static __global__ void __launch_bounds__(128) k_pol_glob_sum(Params p)
 }
 
 // stage sampling (utils.sample, decima/utils.py:19-23) + the rows of the executor-count head
-static __global__ void __launch_bounds__(128) k_pol_sample_stage(Params p, const int32_t *forced_stage)
+// streams: DEVICE u32[B], each env's policy sampling stream (ssb_set_policy_streams), the Philox counter's second word
+static __global__ void __launch_bounds__(128)
+k_pol_sample_stage(Params p, const int32_t *forced_stage, const uint32_t *streams)
 {
     const int b = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (b >= p.B) return;
@@ -682,7 +684,7 @@ static __global__ void __launch_bounds__(128) k_pol_sample_stage(Params p, const
     const int N = live ? oh.num_nodes : 0, Ja = live ? oh.num_active_jobs : 0;
     const int n_cand = live ? p.pl_ncand[b] : 0;
     const EnvHdr &h = p.hdr[b];
-    const uint4 rw = philox4x32_10(h.policy_draws, 0u, 4u, 0u, (uint32_t)h.seed, (uint32_t)(h.seed >> 32));
+    const uint4 rw = philox4x32_10(h.policy_draws, streams[b], 4u, 0u, (uint32_t)h.seed, (uint32_t)(h.seed >> 32));
     const float u1 = ((float)(rw.x >> 8) + 0.5f) * (1.0f / 16777216.0f);
     float lgprob = 0.0f, h_stage = 0.0f;
     const int stage_idx = n_cand > 0 ? sample_w(p.pol_stage_logits + (size_t)b * p.Sc, n_cand,
@@ -722,7 +724,7 @@ static __global__ void __launch_bounds__(128) k_pol_sample_stage(Params p, const
 
 static __global__ void __launch_bounds__(128)
 k_pol_sample_exec(Params p, const int32_t *forced_num_exec, int32_t *stage_idx_out, int32_t *num_exec_out,
-                  int advance_draws)
+                  int advance_draws, const uint32_t *streams)
 {
     const int b = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (b >= p.B) return;
@@ -731,7 +733,7 @@ k_pol_sample_exec(Params p, const int32_t *forced_num_exec, int32_t *stage_idx_o
     const int job_idx = act[1];
     const int cap = job_idx >= 0 ? p.dec_caps[(size_t)b * p.Jc + job_idx] : 0;
     const uint32_t pd = h.policy_draws;
-    const uint4 rw = philox4x32_10(pd, 0u, 4u, 0u, (uint32_t)h.seed, (uint32_t)(h.seed >> 32));
+    const uint4 rw = philox4x32_10(pd, streams[b], 4u, 0u, (uint32_t)h.seed, (uint32_t)(h.seed >> 32));
     const float u2 = ((float)(rw.y >> 8) + 0.5f) * (1.0f / 16777216.0f);
     float lgprob = p.pol_lgprob[b], h_exec = 0.0f;
     int num_exec = 0;

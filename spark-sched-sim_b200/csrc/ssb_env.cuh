@@ -97,6 +97,17 @@ struct BankDev {
 // batches, e.g. the single-env facade), or round 1's shared-memory tf32 tiles (kept for A/B measurements).
 enum { POLICY_TILES = 0, POLICY_FUSED = 1, POLICY_TILES_TF32 = 2 };
 
+// The stored-observation buffers ssb_decima_attach_rollout_store hands the Decima rollouts (snap == nullptr: none)
+struct RolloutStore {
+    char *snap;  // [cap] ssb_decima_snapshot blocks
+    int32_t cap;
+    int32_t *stage_sel, *exec_sel;  // [cap][B]
+    bool operator==(const RolloutStore &o) const
+    {
+        return snap == o.snap && cap == o.cap && stage_sel == o.stage_sel && exec_sel == o.exec_sel;
+    }
+};
+
 struct ssb_env {
     ssb_config cfg;
     Dims dims;
@@ -121,6 +132,7 @@ struct ssb_env {
     ssb_transition *dg_traj;
     int dg_k, dg_events, dg_autoreset, no_graph;
     uint64_t dg_seed_step;
+    RolloutStore dg_store;
     int policy_mode;    // POLICY_* below (SSB_DECIMA_MODE overrides the default)
     void *bw_scratch;   // ssb_decima_attach_backward_scratch
     int bw_saved;       // the last policy evaluation left its levels' input rows in bw_scratch
@@ -128,6 +140,9 @@ struct ssb_env {
     int snap_loaded;    // ssb_decima_snapshot_load: a stored observation is in place, the live one parked
     int auto_reset;     // ssb_set_autoreset
     uint64_t auto_seed_step;
+    // Decima policy unit only (ssb_policy.cu): the simulator kernels never see these
+    uint32_t *pol_streams;  // [B] policy sampling stream of every env (ssb_set_policy_streams), in the workspace
+    RolloutStore store;     // ssb_decima_attach_rollout_store
 };
 
 // ---- internal entry points across the units (C linkage like the public ones; not exported through include/ssb.h)
@@ -139,7 +154,7 @@ int ssb_i_step_launch(ssb_env *env, const int32_t *stage_idx, const int32_t *num
 int ssb_i_decima_obs(ssb_env *env, cudaStream_t s);  // the observation adapter kernel
 int ssb_i_decima_obs_cta(ssb_env *env, cudaStream_t s);  // its one-CTA-per-env version (ssb_policy.cu)
 // ssb_policy.cu
-void ssb_i_policy_carve(Carver &cv, const ssb_config &c, const Dims &d, ssb::Params &p);
+void ssb_i_policy_carve(Carver &cv, const ssb_config &c, const Dims &d, ssb::Params &p, uint32_t **pol_streams);
 int ssb_i_policy_init(ssb_env *env);
 void ssb_i_drop_decision_graph(ssb_env *env);
 }

@@ -81,7 +81,7 @@ __global__ void k_traj_post(Params p, ssb_transition *traj, int K)
 
 }  // namespace
 
-void ssb_i_policy_carve(Carver &cv, const ssb_config &c, const Dims &d, Params &p)
+void ssb_i_policy_carve(Carver &cv, const ssb_config &c, const Dims &d, Params &p, uint32_t **pol_streams)
 {
     const size_t B = c.num_envs;
     {
@@ -133,6 +133,7 @@ void ssb_i_policy_carve(Carver &cv, const ssb_config &c, const Dims &d, Params &
         p.as_kind = cv.take<uint8_t>(B);
         p.as_fresh = cv.take<uint8_t>(B);
         p.as_any = cv.take<int32_t>(4);
+        *pol_streams = cv.take<uint32_t>(B);
     }
 }
 
@@ -225,6 +226,7 @@ int ssb_i_policy_init(ssb_env *env)
     const Dims &d = env->dims;
     Params &p = env->p;
     (void)p;
+    CUDA_TRY(cudaMemset(env->pol_streams, 0, sizeof(uint32_t) * (size_t)cfg->num_envs));  // stream 0 for every env
     {
         env->policy_mode = cfg->num_envs <= 2 * env->num_sms ? POLICY_FUSED : POLICY_TILES;
         if (const char *pm = getenv("SSB_DECIMA_MODE")) env->policy_mode = std::max(0, std::min(atoi(pm), 2));
@@ -343,7 +345,7 @@ static int decima_policy_impl(ssb_env *env, const int32_t *forced_stage, const i
         // the whole decision of every env in one persistent kernel (ssb_decima_fused.cuh)
         CUDA_TRY(cudaMemsetAsync(p.fz_cursor, 0, sizeof(int32_t) * 4, s));
         fz::fused::Args a{forced_stage, forced_num_exec, stage_idx_out, num_exec_out, p.fz_cursor,
-                          run_adapter ? 1 : 0, advance_draws ? 1 : 0, env->fused_group};
+                          run_adapter ? 1 : 0, advance_draws ? 1 : 0, env->fused_group, env->pol_streams};
         const int groups = (p.B + env->fused_group - 1) / env->fused_group;
         fz::fused::k_decima_fused<<<std::min(groups, 2 * env->num_sms), fz::fused::THREADS, fz::fused::Smem::BYTES, s>>>(p, a);
         CUDA_TRY(cudaGetLastError());
@@ -384,10 +386,10 @@ static int decima_policy_impl(ssb_env *env, const int32_t *forced_stage, const i
     // (score heads: four CTAs per SM in the TMEM path; round 1's shared-memory tiles fit one)
     const int head_ctas = env->policy_mode == POLICY_TILES_TF32 ? 1 : 4;
     if ((rc = launch_tile<tc::ST_STAGE>(env, nullptr, nullptr, cnt + tc::CNT_CAND, 0, head_ctas, s))) return rc;
-    tc::k_pol_sample_stage<<<warp_grid, 128, 0, s>>>(p, forced_stage);
+    tc::k_pol_sample_stage<<<warp_grid, 128, 0, s>>>(p, forced_stage, env->pol_streams);
     if ((rc = launch_tile<tc::ST_EXEC>(env, p.pl_exec, nullptr, cnt + tc::CNT_EXEC, 0, head_ctas, s))) return rc;
     tc::k_pol_sample_exec<<<warp_grid, 128, 0, s>>>(p, forced_num_exec, stage_idx_out, num_exec_out,
-                                                    advance_draws ? 1 : 0);
+                                                    advance_draws ? 1 : 0, env->pol_streams);
     CUDA_TRY(cudaGetLastError());
     SSB_MARK(env, s);
     return SSB_OK;
@@ -448,6 +450,19 @@ struct GatherParts {
     size_t off[8];      // byte offset of each part inside a snapshot block
     size_t stride[8];   // bytes per environment
 };
+GatherParts gather_parts(const ssb_env *env)
+{
+    SnapPart parts[8];
+    snapshot_parts(env, parts);
+    GatherParts gp;
+    size_t off = 0;
+    for (int q = 0; q < 8; q++) {
+        gp.off[q] = off;
+        gp.stride[q] = parts[q].bytes / (size_t)env->p.B;
+        off += (parts[q].bytes + 255) & ~size_t(255);
+    }
+    return gp;
+}
 }  // namespace
 __global__ void __launch_bounds__(128)
 k_snapshot_gather(Params p, GatherParts gp, const char *src, size_t block_bytes, int num_steps, const int32_t *src_step,
@@ -487,23 +502,64 @@ k_snapshot_gather(Params p, GatherParts gp, const char *src, size_t block_bytes,
     for (int w = tid; w < sh.num_nodes; w += 128) dm[w] = sm[w];
 }
 
+// The scatter counterpart: env b's live observation -- the one the policy call just sampled its action on -- into slot
+// b of block d of the attached rollout store, and its Decima-format action into [d][b]; only the rows in use are
+// copied.  d = *traj_d (ssb_rollout_decima) or as_rows[b] (ssb_rollout_decima_async).  Rows that will hold no
+// transition are not written: an env outside its duration (async), and in the sync rollout what k_step is about to
+// do instead of a step -- re-seed the env (auto-reset) or idle on a finished episode (k_traj_post flags both 8).
+__global__ void __launch_bounds__(128)
+k_snapshot_scatter(Params p, GatherParts gp, RolloutStore rs, size_t block_bytes, int async, int auto_reset)
+{
+    const int b = blockIdx.x, tid = threadIdx.x;
+    if (b >= p.B) return;
+    const ssb_obs_hdr sh = p.obs_hdr[b];
+    int d;
+    if (async) {
+        if (p.as_kind[b] != 1) return;
+        d = p.as_rows[b];
+    } else {
+        const EnvHdr &h = p.hdr[b];
+        if ((auto_reset && !h.error && (h.done || sh.truncated)) || (h.done && h.error < 1000)) return;
+        d = *p.traj_d;
+    }
+    if (d < 0 || d >= rs.cap) return;  // (the rollouts check their row count against the capacity up front)
+    char *blk = rs.snap + (size_t)d * block_bytes;
+    if (tid == 0) {
+        reinterpret_cast<ssb_obs_hdr *>(blk + gp.off[0])[b] = sh;
+        reinterpret_cast<int32_t *>(blk + gp.off[7])[b] = p.dec_depth[b];
+        rs.stage_sel[(size_t)d * p.B + b] = p.pol_action[(size_t)b * 4];
+        rs.exec_sel[(size_t)d * p.B + b] = p.pol_action[(size_t)b * 4 + 2];
+    }
+    auto copy4 = [&](int part, const void *src, size_t bytes) {  // 4-byte words, as k_snapshot_gather
+        const uint32_t *s = reinterpret_cast<const uint32_t *>(static_cast<const char *>(src) + (size_t)b * gp.stride[part]);
+        uint32_t *dw = reinterpret_cast<uint32_t *>(blk + gp.off[part] + (size_t)b * gp.stride[part]);
+        for (size_t w = tid; w < bytes / 4; w += 128) dw[w] = s[w];
+    };
+    copy4(1, p.obs_edges, (size_t)sh.num_edges * 8);              // edge links
+    copy4(2, p.obs_dag_ptr, ((size_t)sh.num_active_jobs + 1) * 4);  // dag_ptr
+    copy4(3, p.dec_feat, (size_t)sh.num_nodes * 20);             // node features
+    copy4(5, p.dec_caps, (size_t)sh.num_active_jobs * 4);        // commit caps
+    copy4(6, p.dec_edge_bits, (size_t)sh.num_edges * 8);         // per-edge level bits
+    const uint8_t *sm = p.dec_stage_mask + (size_t)b * gp.stride[4];
+    uint8_t *dm = reinterpret_cast<uint8_t *>(blk + gp.off[4] + (size_t)b * gp.stride[4]);
+    for (int w = tid; w < sh.num_nodes; w += 128) dm[w] = sm[w];
+}
+static int store_scatter(ssb_env *env, bool async, cudaStream_t s)
+{
+    if (!env->store.snap) return SSB_OK;
+    k_snapshot_scatter<<<env->p.B, 128, 0, s>>>(env->p, gather_parts(env), env->store, snapshot_bytes(env), async ? 1 : 0,
+                                               env->auto_reset);
+    CUDA_TRY(cudaGetLastError());
+    return SSB_OK;
+}
+
 int ssb_decima_snapshot_gather(ssb_env *env, const void *snapshots, int32_t num_steps, const int32_t *src_step,
                                const int32_t *src_env, void *dst, void *stream)
 {
     if (!env || !snapshots || !src_step || !src_env || !dst || num_steps < 1 || !env->p.dec_feat) return SSB_E_INVALID;
     SSB_ON_DEVICE(env);
     const Params &p = env->p;
-    SnapPart parts[8];
-    const int n = snapshot_parts(env, parts);
-    if (n != 8) return SSB_E_INVALID;
-    GatherParts gp;
-    size_t off = 0;
-    for (int q = 0; q < 8; q++) {
-        gp.off[q] = off;
-        gp.stride[q] = parts[q].bytes / (size_t)p.B;
-        off += (parts[q].bytes + 255) & ~size_t(255);
-    }
-    k_snapshot_gather<<<p.B, 128, 0, (cudaStream_t)stream>>>(p, gp, static_cast<const char *>(snapshots), snapshot_bytes(env),
+    k_snapshot_gather<<<p.B, 128, 0, (cudaStream_t)stream>>>(p, gather_parts(env), static_cast<const char *>(snapshots), snapshot_bytes(env),
                                                              num_steps, src_step, src_env, static_cast<char *>(dst));
     CUDA_TRY(cudaGetLastError());
     SSB_MARK(env, stream);
@@ -786,6 +842,7 @@ static int decima_decision(ssb_env *env, int32_t num_decisions, int32_t max_even
     const int tb = (p.B + 127) / 128;
     int rc = ssb_decima_policy(env, nullptr, nullptr, p.pol_act_a, p.pol_act_n, s);
     if (rc) return rc;
+    if ((rc = store_scatter(env, false, s))) return rc;
     if (traj) k_traj_pre<<<tb, 128, 0, s>>>(p, p.pol_act_a, p.pol_act_n, traj, num_decisions);
     if ((rc = ssb_step(env, p.pol_act_a, p.pol_act_n, nullptr, max_events, s))) return rc;
     if (traj) k_traj_post<<<tb, 128, 0, s>>>(p, traj, num_decisions);
@@ -797,6 +854,7 @@ static int decima_decision(ssb_env *env, int32_t num_decisions, int32_t max_even
 int ssb_rollout_decima(ssb_env *env, int32_t num_decisions, int32_t max_events, ssb_transition *traj, void *stream)
 {
     if (!env || !env->p.pol_w || num_decisions < 0) return SSB_E_INVALID;
+    if (env->store.snap && num_decisions > env->store.cap) return SSB_E_INVALID;
     SSB_ON_DEVICE(env);
     cudaStream_t caller = (cudaStream_t)stream, s = caller;
     // the legacy default stream cannot be captured: run on the handle's own stream, ordered after / before the
@@ -812,7 +870,8 @@ int ssb_rollout_decima(ssb_env *env, int32_t num_decisions, int32_t max_events, 
     // (10-100 us) and strictly dependent, so the per-launch gaps are a visible share of a decision.
     // (SSB_NO_GRAPH=1 launches them one by one.)
     const bool same = env->dg_exec && env->dg_traj == traj && env->dg_k == num_decisions && env->dg_events == max_events &&
-                      env->dg_autoreset == env->auto_reset && env->dg_seed_step == env->auto_seed_step;
+                      env->dg_autoreset == env->auto_reset && env->dg_seed_step == env->auto_seed_step &&
+                      env->dg_store == env->store;
     if (!same && !env->no_graph) {
         if (env->dg_exec) { cudaGraphExecDestroy(env->dg_exec); env->dg_exec = nullptr; }
         cudaGraph_t g = nullptr;
@@ -829,6 +888,7 @@ int ssb_rollout_decima(ssb_env *env, int32_t num_decisions, int32_t max_events, 
             if (ie != cudaSuccess) { env->dg_exec = nullptr; env->no_graph = 1; cudaGetLastError(); }
             env->dg_traj = traj; env->dg_k = num_decisions; env->dg_events = max_events;
             env->dg_autoreset = env->auto_reset; env->dg_seed_step = env->auto_seed_step;
+            env->dg_store = env->store;
         }
     }
     for (int d = 0; d < num_decisions; d++) {
@@ -889,6 +949,7 @@ int ssb_rollout_decima_async(ssb_env *env, int32_t max_decisions, double rollout
                              ssb_transition *traj, int32_t *num_steps, double *elapsed, void *stream)
 {
     if (!env || !env->p.pol_w || max_decisions < 1 || !(rollout_duration > 0.0) || !traj) return SSB_E_INVALID;
+    if (env->store.snap && max_decisions > env->store.cap) return SSB_E_INVALID;
     SSB_ON_DEVICE(env);
     cudaStream_t s = (cudaStream_t)stream;
     const Params &p = env->p;
@@ -904,6 +965,7 @@ int ssb_rollout_decima_async(ssb_env *env, int32_t max_decisions, double rollout
             k_dasync_begin<<<tb, 128, 0, s>>>(p, rollout_duration, max_decisions);
             int rc = decima_policy_impl(env, nullptr, nullptr, p.pol_act_a, p.pol_act_n, true, true, s, p.as_kind);
             if (rc) return rc;
+            if ((rc = store_scatter(env, true, s))) return rc;
             k_dasync_pre<<<tb, 128, 0, s>>>(p, p.pol_act_a, p.pol_act_n, traj, max_decisions);
             // mask = as_kind (0: untouched); finished episodes are re-seeded with seed + seed_step * reset_count
             if ((rc = ssb_i_step_launch(env, p.pol_act_a, p.pol_act_n, p.as_kind, 0, nullptr, nullptr, 0, s, 1, seed_step))) return rc;
@@ -917,6 +979,31 @@ int ssb_rollout_decima_async(ssb_env *env, int32_t max_decisions, double rollout
     if (num_steps) CUDA_TRY(cudaMemcpyAsync(num_steps, p.as_rows, sizeof(int32_t) * (size_t)p.B, cudaMemcpyDeviceToDevice, s));
     if (elapsed) CUDA_TRY(cudaMemcpyAsync(elapsed, p.as_elapsed, sizeof(double) * (size_t)p.B, cudaMemcpyDeviceToDevice, s));
     SSB_MARK(env, s);
+    return SSB_OK;
+}
+
+int ssb_decima_attach_rollout_store(ssb_env *env, void *snapshots, int32_t capacity, int32_t *stage_sel, int32_t *exec_sel)
+{
+    if (!env || !env->p.pol_w) return SSB_E_INVALID;
+    if (!snapshots) {
+        env->store = RolloutStore{};
+        return SSB_OK;
+    }
+    if (env->snap_loaded || capacity < 1 || !stage_sel || !exec_sel) return SSB_E_INVALID;
+    env->store = RolloutStore{static_cast<char *>(snapshots), capacity, stage_sel, exec_sel};
+    return SSB_OK;
+}
+
+int ssb_set_policy_streams(ssb_env *env, const uint32_t *streams)
+{
+    if (!env || !env->p.pol_w) return SSB_E_INVALID;
+    CUDA_TRY(cudaSetDevice(env->device));
+    // policy calls already enqueued sample with the streams they were enqueued with
+    CUDA_TRY(cudaDeviceSynchronize());
+    const size_t n = sizeof(uint32_t) * (size_t)env->p.B;
+    if (streams) CUDA_TRY(cudaMemcpy(env->pol_streams, streams, n, cudaMemcpyHostToDevice));
+    else CUDA_TRY(cudaMemset(env->pol_streams, 0, n));
+    CUDA_TRY(cudaDeviceSynchronize());
     return SSB_OK;
 }
 

@@ -1,9 +1,11 @@
 """The reference's PPO trainer (trainers/ppo.py) on the device: the loss head (`_compute_loss`, :104-140: forward values
 and the adjoint seeds d loss / d lgprob, d loss / d entropy for the policy's backward pass), the parameter update
 (clip_grad_norm_ + Adam), the rollout store and `_train`'s epoch loop over shuffled mini-batches of samples."""
+import numpy as np
 import torch
 
 from . import _native as nat
+from . import parallel
 from .returns import _stream
 
 
@@ -155,7 +157,9 @@ class RolloutStore:
     """RolloutBuffer (trainers/rollout_worker.py:18-46) of ALL environments of a handle for K decisions, on the device:
     per decision k the stored observations of the B envs (one ssb_decima_snapshot block), the Decima-format actions,
     their log-probabilities, rewards, wall times and which (k, b) hold a real transition.  `collect` is the rollout
-    loop { snapshot ; policy ; step } (rollout_worker.py:135-157) with the sampled policy."""
+    loop { snapshot ; policy ; step } (rollout_worker.py:135-157) with the sampled policy, one decision per call;
+    `collect_fused` runs the device's Decima rollouts, which write the observations themselves, and also keeps the
+    transition rows that ReturnsCalculator / Baseline read (`traj`, `num_steps`, `final_wall`)."""
 
     def __init__(self, env, num_decisions: int):
         self.env, self.K, self.B = env, int(num_decisions), env.num_envs
@@ -167,6 +171,7 @@ class RolloutStore:
         self.reward = torch.zeros(self.K, self.B, dtype=torch.float64, device=dev)
         self.wall_time = torch.zeros(self.K + 1, self.B, dtype=torch.float64, device=dev)
         self.valid = torch.zeros(self.K, self.B, dtype=torch.bool, device=dev)
+        self.traj = self.num_steps = self.final_wall = None  # set by collect_fused
 
     def samples(self, idx: torch.Tensor):
         """The stored observations of dataset indices idx (= k * B + b, at most B of them) for
@@ -206,6 +211,67 @@ class RolloutStore:
             self.reward[k] = torch.from_numpy(h1["reward"].copy()).to(env.device)
         self.wall_time[self.K] = torch.from_numpy(env.hdr()["wall_time"].copy()).to(env.device)
         return self
+
+    def collect_fused(self, rollout_duration=None, seed_step=1, max_events=0):
+        """The store filled by the device's Decima rollouts, without a host round trip per decision.
+        rollout_duration None: RolloutWorkerSync (rollout_worker.py:135-157) -- the caller has reset the envs and
+        auto-reset is off; rollout_decima(K) runs, a finished env idles, so each env's transitions are its rows
+        [0, num_steps) and final_wall is its header's wall time.  Otherwise RolloutWorkerAsync (:160-206):
+        rollout_decima_async(K, rollout_duration, seed_step), final_wall = the accumulated time.  `traj` (the
+        transition rows, ssb_transition[B][K]), `num_steps` (i32[B]) and `final_wall` (f64[B]) are what
+        ReturnsCalculator and Baseline take."""
+        env, K, B = self.env, self.K, self.B
+        if rollout_duration is None:
+            assert not env._settings.get("autoreset", (False,))[0], "the sync protocol runs with auto-reset off"
+            traj = env.rollout_decima(K, max_events=max_events, store=self)
+            valid = (traj.view(torch.int32).view(B, K, 8)[..., 6] & 8) == 0
+            num_steps = valid.sum(1, dtype=torch.int32)
+            off = nat.OBS_HDR_DTYPE.fields["wall_time"][1]
+            final_wall = env.hdr_bytes[:, off:off + 8].contiguous().view(torch.float64).reshape(B)
+        else:
+            traj, num_steps, final_wall = env.rollout_decima_async(K, rollout_duration, seed_step, store=self)
+            valid = torch.arange(K, device=env.device)[None, :] < num_steps[:, None]
+        rows64 = traj.view(torch.float64).view(B, K, 4)
+        self.valid.copy_(valid.t())
+        self.lgprob.copy_(traj.view(torch.float32).view(B, K, 8)[..., 7].t())
+        self.reward.copy_(rows64[..., 1].t())
+        self.wall_time[:K] = rows64[..., 0].t()
+        self.wall_time[K] = final_wall
+        self.traj, self.num_steps, self.final_wall = traj, num_steps, final_wall
+        return self
+
+
+def rollout_groups(num_sequences, num_rollouts, seed, rank=0, world=1):
+    """The reference trainer's `num_sequences x num_rollouts` rollout workers (trainer.py:264-293) as this rank's share
+    of the envs of BatchedSparkSchedSimEnv handles: worker i (global index) plays the job sequence of seed
+    seed + i // num_rollouts and samples its actions from policy stream i % num_rollouts (set_policy_streams), so the
+    members of a group share the arrivals but not the actions.  Returns (seeds u64[n], streams u32[n], seed_step =
+    num_sequences: the k-th episode of every member of group j is seeded seed + j + num_sequences * k).  A rank holds
+    whole groups (Baseline averages within a group), n = num_sequences * num_rollouts / world."""
+    total = num_sequences * num_rollouts
+    n, rem = divmod(total, world)
+    assert rem == 0 and n % num_rollouts == 0, "every rank must hold whole groups of num_rollouts envs"
+    seeds, seed_step = parallel.reference_worker_seeds(seed, num_sequences, num_rollouts)
+    i = np.arange(rank * n, (rank + 1) * n)
+    return seeds[i], (i % num_rollouts).astype(np.uint32), seed_step
+
+
+def train_iteration(env, store, returns_calc, baseline, loss_fn: PPOLoss, adam: Adam, num_epochs, num_batches, target_kl,
+                    allreduce=None, generator=None):
+    """One iteration of the reference trainer after collection (trainer.py:172-212 _preprocess_rollouts +
+    PPO.train_on_rollouts) on a store filled by RolloutStore.collect_fused: returns_calc (ReturnsCalculator) and
+    baseline (Baseline) on the store's transition rows, transposed to the store's [K, B] layout, then
+    ppo_train_samples.  Returns ppo_train_samples' summary plus "collect_stats" (the statistics of this handle's envs,
+    parallel.stats_from_sums) and the "returns" / "baselines" (f64 [B, K] device tensors) it trained on."""
+    assert store.traj is not None, "fill the store with collect_fused first"
+    returns = returns_calc(store.traj, store.num_steps, store.final_wall, store.K)
+    baselines = baseline(store.traj, returns, store.num_steps)
+    summary = ppo_train_samples(env, store, returns.t().contiguous(), baselines.t().contiguous(), loss_fn, adam,
+                                num_epochs=num_epochs, num_batches=num_batches, target_kl=target_kl,
+                                allreduce=allreduce, generator=generator)
+    summary["collect_stats"] = parallel.stats_from_sums(env.collect_stats())
+    summary["returns"], summary["baselines"] = returns, baselines
+    return summary
 
 
 def _evaluate_slots(env, store, staging, ks, bs):
