@@ -1,5 +1,6 @@
-"""Development aid: the fused policy kernel against round 1's list-driven tile path on the same states (two handles
-driven with the same actions); prints the first step / environments where candidates, actions or scores differ."""
+"""Development aid: the fused policy kernel (MODE_A, default 1) against the list-driven tile path (MODE_B, default 0) on
+the same states (two handles driven with the same actions); prints the first step / environments where candidates,
+actions or scores differ."""
 import os
 import os.path as osp
 import sys
@@ -21,7 +22,7 @@ cfg = {"num_executors": 10, "job_arrival_cap": 8, "job_arrival_rate": 4.0e-5, "m
 z = np.load(osp.join(REPO, "tests", "golden", "decima_model.npz"))
 envs = []
 for tiles in (0, 1):
-    os.environ["SSB_DECIMA_MODE"] = str(int(os.environ.get("MODE_B", "2")) if tiles else int(os.environ.get("MODE_A", "1")))
+    os.environ["SSB_DECIMA_MODE"] = str(int(os.environ.get("MODE_B", "0")) if tiles else int(os.environ.get("MODE_A", "1")))
     e = BatchedSparkSchedSimEnv(cfg, num_envs=B, bank=synthetic_bank(0), max_jobs=10, tape_capacity=len(tr["tape"]) + 8,
                                 decima_policy=True)
     e.set_decima_weights({k: z[k] for k in z.files})

@@ -1,5 +1,5 @@
 """One Decima policy call at mid-episode (decision 60) inside a cudaProfilerStart/Stop range, for
-    ncu --profile-from-start off --set full --import-source on -k regex:k_tile_mlp ... python profiles/policy_ncu_target.py"""
+    ncu --profile-from-start off --set full --import-source on -k regex:k_tile3 ... python profiles/policy_ncu_target.py"""
 import os.path as osp
 import sys
 

@@ -1,9 +1,9 @@
-import sys, os.path as osp
+import os, sys, os.path as osp
 sys.path.insert(0, '.'); sys.path.insert(0, 'tests')
 import numpy as np, torch
 from spark_sched_sim_b200.batched_env import BatchedSparkSchedSimEnv
 cfg = {"num_executors": 10, "job_arrival_cap": 50, "job_arrival_rate": 4.0e-5, "moving_delay": 2000.0, "warmup_delay": 1000.0}
-B = 4096
+B = int(os.environ.get("POLICY_B", "4096"))  # 4096: mode 0 by default; up to 2 x SMs envs: mode 1
 env = BatchedSparkSchedSimEnv(cfg, num_envs=B, decima_policy=True)
 z = np.load(osp.join('tests', 'golden', 'decima_model.npz'))
 env.set_decima_weights({k: z[k] for k in z.files})

@@ -3,14 +3,17 @@ touch its kernels:
 
     nvcc -cubin -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -fmad=false \\
          -o new.cubin spark-sched-sim_b200/csrc/ssb_api.cu        (same for the parent commit -> old.cubin)
-    python profiles/sass_compare.py old.cubin new.cubin
+    python profiles/sass_compare.py [--mask-cbank] old.cubin new.cubin
 
 Normalisation: `cuobjdump -sass`, the instruction text of each function (addresses, encodings and comments dropped),
 and the hash nvcc puts into the anonymous-namespace part of mangled names masked (it depends on the file's path).
+--mask-cbank also masks the offsets of constant-bank 0 operands (`c[0x0][0x...]`): where the kernel arguments sit
+there, which moves when a struct passed by value (Params) changes size while the code does not.
 Prints one line per function (instruction count, digest, identical / DIFFERENT / only in one) and exits 1 unless
 every function is identical in both."""
 from __future__ import annotations
 
+import argparse
 import hashlib
 import re
 import subprocess
@@ -19,7 +22,7 @@ import sys
 CUOBJDUMP = "/usr/local/cuda/bin/cuobjdump"
 
 
-def normalised_sass(cubin: str) -> dict[str, list[str]]:
+def normalised_sass(cubin: str, mask_cbank: bool = False) -> dict[str, list[str]]:
     out = subprocess.run([CUOBJDUMP, "-sass", cubin], capture_output=True, text=True, check=True).stdout
     funcs: dict[str, list[str]] = {}
     cur = None
@@ -31,12 +34,13 @@ def normalised_sass(cubin: str) -> dict[str, list[str]]:
             continue
         m = re.match(r"\s*/\*[0-9a-f]{4,}\*/\s+(.*?)\s*;", line)
         if m and cur is not None:
-            cur.append(m.group(1))
+            ins = m.group(1)
+            cur.append(re.sub(r"c\[0x0\]\[0x[0-9a-f]+\]", "c[0x0][CB]", ins) if mask_cbank else ins)
     return funcs
 
 
-def main(old: str, new: str) -> int:
-    a, b = normalised_sass(old), normalised_sass(new)
+def main(old: str, new: str, mask_cbank: bool = False) -> int:
+    a, b = normalised_sass(old, mask_cbank), normalised_sass(new, mask_cbank)
     same = True
     for name in sorted(set(a) | set(b)):
         if name not in a or name not in b:
@@ -53,4 +57,9 @@ def main(old: str, new: str) -> int:
 
 
 if __name__ == "__main__":
-    sys.exit(main(sys.argv[1], sys.argv[2]))
+    ap = argparse.ArgumentParser(description="kernel-by-kernel SASS comparison of two cubins")
+    ap.add_argument("old")
+    ap.add_argument("new")
+    ap.add_argument("--mask-cbank", action="store_true", help="ignore the offsets of constant-bank 0 operands")
+    args = ap.parse_args()
+    sys.exit(main(args.old, args.new, args.mask_cbank))

@@ -111,15 +111,6 @@ k_rollout_fair_async(Params p, int max_decisions, double duration, int dynamic_p
         max_decisions, duration, seed_step, traj, num_steps, elapsed_out);
 }
 
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32) k_decima_obs(Params p)
-{
-    __shared__ uint64_t Sk[WARPS_PER_CTA][64];
-    const int b = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (b >= p.B) return;
-    Sim sim(p, b, lane);
-    sim.decima_obs_w(Sk[threadIdx.x >> 5]);
-}
-
 // collect_stats sums in a fixed order: block k reduces the envs k, k + STATS_BLOCKS, ... (one warp per env, lanes
 // over its jobs) into part[k][6]; a last warp adds the blocks' partial sums in block order.
 constexpr int STATS_BLOCKS = 128;
@@ -749,16 +740,6 @@ int ssb_decima_obs(ssb_env *env, void *stream)
     const int rc = ssb_i_decima_obs(env, (cudaStream_t)stream);
     if (rc) return rc;
     SSB_MARK(env, stream);
-    return SSB_OK;
-}
-
-int ssb_i_decima_obs(ssb_env *env, cudaStream_t s)
-{
-    // one CTA per env (ssb_policy.cu) unless SSB_DECIMA_ADAPTER=warp asks for the one-warp-per-env kernel (A/B)
-    static const bool warp_version = [] { const char *v = getenv("SSB_DECIMA_ADAPTER"); return v && !strcmp(v, "warp"); }();
-    if (!warp_version) return ssb_i_decima_obs_cta(env, s);
-    k_decima_obs<<<env->grid, WARPS_PER_CTA * 32, 0, s>>>(env->p);
-    CUDA_TRY(cudaGetLastError());
     return SSB_OK;
 }
 

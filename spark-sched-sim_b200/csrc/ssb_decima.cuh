@@ -12,7 +12,7 @@ namespace ssb {
 // ABI layout (dw): the tensors of models/decima/model.pt in state_dict order, each [out][in] row-major
 // (42 tensors, 20 802 floats).  Device layout (dd): per layer the TRANSPOSED weight [in][out] followed
 // by the bias, every tensor padded to a multiple of 4 floats (ssb_set_decima_weights does the re-layout);
-// tc::k_build_blob turns it into the per-stage tf32 hi/lo tiles the tensor-core kernel copies to shared memory.
+// fz::k_build_blob turns it into the per-stage bf16 three-term weight blobs the tensor-core kernels copy to shared memory.
 namespace dw {
 constexpr int mlp(int in, int h1, int h2, int out) { return h1 * in + h1 + h2 * h1 + h2 + out * h2 + out; }
 constexpr int TOTAL = mlp(5, 32, 16, 16) + 2 * mlp(16, 32, 16, 16) + mlp(21, 32, 16, 16) + mlp(16, 32, 16, 16) +

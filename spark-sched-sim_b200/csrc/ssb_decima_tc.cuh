@@ -1,26 +1,16 @@
-// ssb_decima_tc.cuh -- Decima policy forward pass batched ACROSS environments on the 5th-generation
-// tensor cores (tcgen05.mma kind::tf32, accumulators in TMEM).
+// ssb_decima_tc.cuh -- the list-driven Decima policy pass, batched ACROSS environments: row-list planning, the gather /
+// scatter of one row, sampling, the adjoint of the score heads and the CUDA-core backward kernels, plus the tcgen05 /
+// mbarrier PTX wrappers that the tensor-core tile routines of ssb_decima_fused.cuh use.
 //
 // DecimaScheduler.schedule (schedulers/decima/scheduler.py:71-99) evaluates seven small 3-layer MLPs
 // (SURVEY.md App. E).  One environment offers ~16 rows per message-passing level -- far too few for a
 // 128-row UMMA tile -- so the work is organised by MLP instead of by environment: a planning pass
 // turns every environment's observation into flat ROW LISTS (all nodes, sinks, the senders and
 // receivers of every level, jobs, schedulable stages, executor counts), and one generic tile kernel
-// runs "gather 128 rows -> Linear/act/Linear/act/Linear on the tensor cores -> scatter" over a list.
+// runs "gather 128 rows -> Linear/act/Linear/act/Linear on the tensor cores -> scatter" over a list
+// (fz::k_tile3 in ssb_decima_fused.cuh: bf16 three-term split, activations in TMEM).
 // The level loop of NodeEncoder (:214-232) stays the literal sequence (deepest level first, parents
 // OVERWRITE their embedding) -- it is a sequence of launches over all environments at once.
-//
-// fp32 accuracy on tf32 tensor cores: every operand is split x = hi + lo (both rounded to tf32) and
-// a product is accumulated as hi*hi + lo*hi + hi*lo (3 MMAs per k-step, fp32 accumulation in TMEM);
-// the dropped lo*lo term is < 2^-22 relative.  Scores agree with the reference's torch fp32 forward
-// within the same 5e-5 the fp32 CUDA-core kernel was held to (tests/test_gpu_decima_policy.py).
-//
-// Tile kernel (128 threads, thread r <-> tile row r <-> TMEM lane r):
-//   A tile  [128 x K]  and the weights W [N x K] sit in shared memory in the canonical K-major,
-//           no-swizzle UMMA layout: 8-row x 16-byte core matrices, LBO = 128 B between the two
-//           16-byte K chunks of one MMA, SBO = (K/4) * 128 B between 8-row groups;
-//   D       [128 x N] fp32 in TMEM columns [0, N); read back with tcgen05.ld.32x32b (one row per
-//           thread), bias + activation applied in registers, and written as the next layer's A tile.
 #pragma once
 #include "ssb_decima.cuh"
 
@@ -36,22 +26,6 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo_bytes
 {
     return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(lbo_bytes >> 4) << 16) |
            ((uint64_t)(sbo_bytes >> 4) << 32) | (1ull << 46);
-}
-// instruction descriptor (cute::UMMA::InstrDescriptor): D = f32, A = B = tf32, both K-major, dense
-__host__ __device__ constexpr uint32_t umma_idesc_tf32(int M, int N)
-{
-    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                          uint32_t accumulate)
-{
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t"
-        "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
 }
 __device__ __forceinline__ void umma_commit(uint32_t mbar)
 {
@@ -110,13 +84,6 @@ __device__ __forceinline__ void tmem_ld_row(uint32_t taddr, float *v)
 #pragma unroll
     for (int i = 0; i < N; i++) v[i] = __uint_as_float(r[i]);
 }
-// cvt.rna.tf32.f32 (round to nearest, ties away from zero, 10 mantissa bits) on the integer ALU: half an ulp added
-// to the magnitude, low 13 bits cleared -- the same bits for every finite input, and it keeps the conversions off the
-// XU pipe (two per element and layer: 49 % of that pipe's peak in the ncu capture of the message pass).
-__device__ __forceinline__ float to_tf32(float x)
-{
-    return __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xffffe000u);
-}
 
 // ------------------------------------------------------------------ row lists and counters
 // p.pl_cnt layout (int32): list lengths, then per level k: senders at [CNT_LVL + 2k], receivers at
@@ -138,80 +105,6 @@ template <> struct Spec<ST_DAG>   { static constexpr int K0 = 24, IN = 21, H1 = 
 template <> struct Spec<ST_GLOB>  { static constexpr int K0 = 16, IN = 16, H1 = 32, H2 = 16, OUT = 16, W = dd::GLOB;  static constexpr bool TANH = false; };
 template <> struct Spec<ST_STAGE> { static constexpr int K0 = 56, IN = 53, H1 = 64, H2 = 64, OUT = 1,  W = dd::STAGE; static constexpr bool TANH = true; };
 template <> struct Spec<ST_EXEC>  { static constexpr int K0 = 40, IN = 36, H1 = 64, H2 = 64, OUT = 1,  W = dd::EXEC;  static constexpr bool TANH = true; };
-
-template <int ST>
-struct Smem {
-    using S = Spec<ST>;
-    static constexpr int KMAX = S::K0 > S::H1 ? (S::K0 > S::H2 ? S::K0 : S::H2) : (S::H1 > S::H2 ? S::H1 : S::H2);
-    static constexpr int W1 = S::H1 * S::K0, W2 = S::H2 * S::H1, W3 = S::OUT > 1 ? S::OUT * S::H2 : 0;
-    // float offsets
-    static constexpr int A_HI = 0, A_LO = A_HI + 128 * KMAX;
-    static constexpr int W1_HI = A_LO + 128 * KMAX, W1_LO = W1_HI + W1;
-    static constexpr int W2_HI = W1_LO + W1, W2_LO = W2_HI + W2;
-    static constexpr int W3_HI = W2_LO + W2, W3_LO = W3_HI + W3;
-    static constexpr int BIAS = W3_LO + W3;                 // H1 + H2 + max(OUT, 1) biases
-    static constexpr int W3V = BIAS + S::H1 + S::H2 + 16;   // OUT == 1: the last layer's H2 weights
-    static constexpr int CTRL = W3V + (S::OUT > 1 ? 0 : S::H2);  // mbarrier (8 B) + TMEM slot (4 B)
-    static constexpr int FLOATS = CTRL + 4;
-    // [W1_HI, CTRL) is the stage's constant "weight blob": built once per weight upload in global memory
-    // (k_build_blob) in exactly this layout, so a CTA's prologue is one coalesced copy
-    static constexpr int BLOB = CTRL - W1_HI;
-    static constexpr size_t BYTES = (size_t)FLOATS * 4 + 128;  // + slack to align the base to 128 B
-};
-
-// canonical K-major no-swizzle offset (in floats) of element (row, k) of a [rows x K] operand
-__device__ __forceinline__ int canon(int row, int k, int K)
-{
-    return (row >> 3) * (K * 8) + (k >> 2) * 32 + (row & 7) * 4 + (k & 3);
-}
-
-// writes this thread's row of the A tile (hi and lo parts) for a layer with K inputs
-template <int K>
-__device__ __forceinline__ void write_a_row(float *a_hi, float *a_lo, int row, const float *v)
-{
-#pragma unroll
-    for (int c = 0; c < K / 4; c++) {
-        float4 h, l;
-        h.x = to_tf32(v[4 * c]);     l.x = to_tf32(v[4 * c] - h.x);
-        h.y = to_tf32(v[4 * c + 1]); l.y = to_tf32(v[4 * c + 1] - h.y);
-        h.z = to_tf32(v[4 * c + 2]); l.z = to_tf32(v[4 * c + 2] - h.z);
-        h.w = to_tf32(v[4 * c + 3]); l.w = to_tf32(v[4 * c + 3] - h.w);
-        const int off = canon(row, 4 * c, K);
-        *reinterpret_cast<float4 *>(a_hi + off) = h;
-        *reinterpret_cast<float4 *>(a_lo + off) = l;
-    }
-}
-// one Linear layer on the tensor cores: D[128 x N] = A[128 x K] . W[N x K]^T with the 3-term split
-template <int K, int N>
-__device__ __forceinline__ void issue_layer(uint32_t tmem_d, const float *a_hi, const float *a_lo, const float *w_hi,
-                                            const float *w_lo, uint32_t mbar)
-{
-    constexpr uint32_t idesc = umma_idesc_tf32(128, N);
-    constexpr uint32_t sbo = (K / 4) * 128;
-    const uint32_t ah = smem_u32(a_hi), al = smem_u32(a_lo), wh = smem_u32(w_hi), wl = smem_u32(w_lo);
-#pragma unroll
-    for (int ks = 0; ks < K / 8; ks++) {
-        const uint64_t dah = umma_desc(ah + ks * 256, 128, sbo), dal = umma_desc(al + ks * 256, 128, sbo);
-        const uint64_t dwh = umma_desc(wh + ks * 256, 128, sbo), dwl = umma_desc(wl + ks * 256, 128, sbo);
-        umma_tf32(tmem_d, dah, dwh, idesc, ks > 0 ? 1u : 0u);
-        umma_tf32(tmem_d, dal, dwh, idesc, 1u);
-        umma_tf32(tmem_d, dah, dwl, idesc, 1u);
-    }
-    umma_commit(mbar);
-}
-// loads a Linear's weight (dd layout: transposed [in][out], then the bias) into the canonical hi/lo tiles
-template <int IN, int K, int N>
-__device__ __forceinline__ void load_weights(const float *__restrict__ wt, float *w_hi, float *w_lo, float *bias, int tid)
-{
-    for (int i = tid; i < N * K; i += 128) {
-        const int n = i / K, k = i % K;
-        const float x = k < IN ? __ldg(wt + k * N + n) : 0.0f;
-        const float h = to_tf32(x);
-        w_hi[canon(n, k, K)] = h;
-        w_lo[canon(n, k, K)] = to_tf32(x - h);
-    }
-    for (int i = tid; i < N; i += 128) bias[i] = __ldg(wt + dd::pad4(IN * N) + i);
-}
 
 struct TileArgs {
     const int32_t *list;    // row ids (base of the array)
@@ -354,177 +247,6 @@ __device__ __forceinline__ float act_tc(float x)
     if (TANH) return tanhf(x);
     return x > 0.0f ? x : 0.2f * x;
 }
-
-// ------------------------------------------------------------------ the tile kernel
-// offset (floats) of stage ST's weight blob in p.pol_wblob
-__host__ __device__ constexpr int blob_size(int st)
-{
-    return st == ST_PREP ? Smem<ST_PREP>::BLOB : st == ST_SINK ? Smem<ST_SINK>::BLOB : st == ST_MSG ? Smem<ST_MSG>::BLOB
-         : st == ST_RCV ? Smem<ST_RCV>::BLOB : st == ST_DAG ? Smem<ST_DAG>::BLOB : st == ST_GLOB ? Smem<ST_GLOB>::BLOB
-         : st == ST_STAGE ? Smem<ST_STAGE>::BLOB : Smem<ST_EXEC>::BLOB;
-}
-__host__ __device__ constexpr int blob_offset(int st)
-{
-    int off = 0;
-    for (int i = 0; i < st; i++) off += blob_size(i);
-    return off;
-}
-constexpr int BLOB_TOTAL = blob_offset(ST_EXEC) + blob_size(ST_EXEC);
-
-// one CTA per stage: dd-layout weights -> canonical hi/lo tiles + biases (+ last-layer vector) in global memory
-template <int ST>
-__global__ void __launch_bounds__(128) k_build_blob(Params p)
-{
-    using S = Spec<ST>;
-    using L = Smem<ST>;
-    const int tid = threadIdx.x;
-    float *sm = p.pol_wblob + blob_offset(ST) - L::W1_HI;  // so that the Smem<ST> offsets apply unchanged
-    float *bias = sm + L::BIAS;
-    const float *w = p.pol_w + S::W;
-    load_weights<S::IN, S::K0, S::H1>(w, sm + L::W1_HI, sm + L::W1_LO, bias, tid);
-    load_weights<S::H1, S::H1, S::H2>(w + dd::layer(S::IN, S::H1), sm + L::W2_HI, sm + L::W2_LO, bias + S::H1, tid);
-    if constexpr (S::OUT > 1) {
-        load_weights<S::H2, S::H2, S::OUT>(w + dd::layer(S::IN, S::H1) + dd::layer(S::H1, S::H2), sm + L::W3_HI,
-                                           sm + L::W3_LO, bias + S::H1 + S::H2, tid);
-    } else {
-        const float *w3 = w + dd::layer(S::IN, S::H1) + dd::layer(S::H1, S::H2);  // [H2][1] then the bias
-        for (int i = tid; i < S::H2; i += 128) sm[L::W3V + i] = __ldg(w3 + i);
-        if (tid == 0) bias[S::H1 + S::H2] = __ldg(w3 + dd::pad4(S::H2));
-    }
-}
-
-#ifdef SSB_PROFILE
-#define TC_STAMP(i) do { if (blockIdx.x == 0 && threadIdx.x == 0) p.prof[ST * 16 + (i)] = (unsigned long long)clock64(); } while (0)
-#else
-#define TC_STAMP(i) do { } while (0)
-#endif
-
-// One 128-row tile through the stage's three layers.  wb = the stage's weight blob in shared memory
-// (layout of Smem<ST> from W1_HI on), a_hi / a_lo = the A tile, tmem = this CTA's 64 accumulator columns.
-template <int ST, bool STAMPS>
-__device__ __forceinline__ void run_tile(const Params &p, const TileArgs &a, const int32_t *list, int n_rows, int tile,
-                                         float *a_hi, float *a_lo, const float *wb, uint32_t mbar, uint32_t tmem,
-                                         uint32_t &parity)
-{
-    using S = Spec<ST>;
-    using L = Smem<ST>;
-    const int tid = threadIdx.x, warp = tid >> 5;
-    const float *bias = wb + (L::BIAS - L::W1_HI);
-    const uint32_t trow = tmem + ((uint32_t)(warp * 32) << 16);  // this warp's 32 TMEM lanes
-        const int row = tile * 128 + tid;
-        int id = -1;
-        if (row < n_rows) id = (ST == ST_STAGE) ? row : list[row];
-        {
-            float in[S::K0];
-            gather_row<ST>(p, a, id, in);
-            if constexpr (ST == ST_MSG || ST == ST_RCV) {
-                const int pos = (a.offset ? *a.offset : 0) + row;
-                if (a.x_save && id >= 0 && pos < a.x_cap) st16(a.x_save + (size_t)pos * 16, *reinterpret_cast<float(*)[16]>(in));
-            }
-            if (STAMPS && tile == (int)blockIdx.x) TC_STAMP(3);
-            write_a_row<S::K0>(a_hi, a_lo, tid, in);
-        }
-        fence_async_smem();
-        __syncthreads();
-        if (STAMPS && tile == (int)blockIdx.x) TC_STAMP(4);
-        if (tid == 0) {
-            tc_fence_after();
-            issue_layer<S::K0, S::H1>(tmem, a_hi, a_lo, wb + (L::W1_HI - L::W1_HI), wb + (L::W1_LO - L::W1_HI), mbar);
-        }
-        mbar_wait(mbar, parity);
-        parity ^= 1;
-        tc_fence_after();
-        if (STAMPS && tile == (int)blockIdx.x) TC_STAMP(5);
-        {
-            float v[S::H1];
-            tmem_ld_row<S::H1>(trow, v);
-#pragma unroll
-            for (int i = 0; i < S::H1; i++) v[i] = act_tc<S::TANH>(v[i] + bias[i]);
-            write_a_row<S::H1>(a_hi, a_lo, tid, v);
-        }
-        tc_fence_before();
-        fence_async_smem();
-        __syncthreads();
-        if (STAMPS && tile == (int)blockIdx.x) TC_STAMP(6);
-        if (tid == 0) {
-            tc_fence_after();
-            issue_layer<S::H1, S::H2>(tmem, a_hi, a_lo, wb + (L::W2_HI - L::W1_HI), wb + (L::W2_LO - L::W1_HI), mbar);
-        }
-        mbar_wait(mbar, parity);
-        parity ^= 1;
-        tc_fence_after();
-        if (STAMPS && tile == (int)blockIdx.x) TC_STAMP(7);
-        float v2[S::H2];
-        tmem_ld_row<S::H2>(trow, v2);
-#pragma unroll
-        for (int i = 0; i < S::H2; i++) v2[i] = act_tc<S::TANH>(v2[i] + bias[S::H1 + i]);
-        if constexpr (S::OUT > 1) {
-            write_a_row<S::H2>(a_hi, a_lo, tid, v2);
-            tc_fence_before();
-            fence_async_smem();
-            __syncthreads();
-            if (tid == 0) {
-                tc_fence_after();
-                issue_layer<S::H2, S::OUT>(tmem, a_hi, a_lo, wb + (L::W3_HI - L::W1_HI), wb + (L::W3_LO - L::W1_HI), mbar);
-            }
-            mbar_wait(mbar, parity);
-            parity ^= 1;
-            tc_fence_after();
-            float o[S::OUT];
-            tmem_ld_row<S::OUT>(trow, o);
-#pragma unroll
-            for (int i = 0; i < S::OUT; i++) o[i] += bias[S::H1 + S::H2 + i];
-            scatter_row<ST>(p, id, o);
-        } else {
-            // score heads end in a single neuron: a dot product in this row's thread
-            float s = bias[S::H1 + S::H2];
-#pragma unroll
-            for (int i = 0; i < S::H2; i++) s = fmaf(wb[L::W3V - L::W1_HI + i], v2[i], s);
-            scatter_row<ST>(p, id, &s);
-        }
-        tc_fence_before();  // this tile's TMEM reads are ordered before the next tile's first MMA
-        if (STAMPS && tile == (int)blockIdx.x) TC_STAMP(8);
-    }
-
-template <int ST>
-__global__ void __launch_bounds__(128) k_tile_mlp(Params p, TileArgs a)
-{
-    using S = Spec<ST>;
-    using L = Smem<ST>;
-    TC_STAMP(0);
-    const int n_rows = *a.count;
-    if (n_rows <= 0) return;
-    const int32_t *list = a.list + (a.offset ? *a.offset : 0);
-    const int n_tiles = (n_rows + 127) >> 7;
-    if ((int)blockIdx.x >= n_tiles) return;
-    extern __shared__ unsigned char smem_raw[];
-    float *sm = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(smem_raw) + 127) & ~uintptr_t(127));
-    const int tid = threadIdx.x, warp = tid >> 5;
-    float *a_hi = sm + L::A_HI, *a_lo = sm + L::A_LO;
-    const uint32_t mbar = smem_u32(sm + L::CTRL), slot = smem_u32(sm + L::CTRL + 2);
-    {
-        const float4 *src = reinterpret_cast<const float4 *>(p.pol_wblob + blob_offset(ST));
-        float4 *dst = reinterpret_cast<float4 *>(sm + L::W1_HI);
-        for (int i = tid; i < L::BLOB / 4; i += 128) dst[i] = __ldg(src + i);
-    }
-    TC_STAMP(1);
-    if (warp == 0) tmem_alloc(slot, 64);
-    if (tid == 0) mbar_init(mbar, 1);
-    fence_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *reinterpret_cast<volatile uint32_t *>(sm + L::CTRL + 2);
-    uint32_t parity = 0;
-    TC_STAMP(2);
-
-    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x)
-        run_tile<ST, true>(p, a, list, n_rows, tile, a_hi, a_lo, sm + L::W1_HI, mbar, tmem, parity);
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, 64);
-    TC_STAMP(9);
-}
-
 
 // ------------------------------------------------------------------ planning kernels (one warp per env)
 // Pass A: per-node level bit sets (which levels a node sends / receives at), row_start, the lists of

@@ -93,9 +93,9 @@ struct BankDev {
 
 
 // How ssb_decima_policy runs: row lists + one launch per MLP pass with the TMEM-resident bf16 three-term tiles (the
-// default for large batches), the whole decision of a group of envs in one persistent kernel (one launch: small
-// batches, e.g. the single-env facade), or round 1's shared-memory tf32 tiles (kept for A/B measurements).
-enum { POLICY_TILES = 0, POLICY_FUSED = 1, POLICY_TILES_TF32 = 2 };
+// default for large batches), or the whole decision of a group of envs in one persistent kernel (one launch: small
+// batches, e.g. the single-env facade).
+enum { POLICY_TILES = 0, POLICY_FUSED = 1 };
 
 // The stored-observation buffers ssb_decima_attach_rollout_store hands the Decima rollouts (snap == nullptr: none)
 struct RolloutStore {
@@ -151,9 +151,8 @@ extern "C" {
 int ssb_i_step_launch(ssb_env *env, const int32_t *stage_idx, const int32_t *num_exec, const uint8_t *mask,
                       int32_t max_events, int32_t *next_a, int32_t *next_n, int dyn, cudaStream_t s,
                       int force_autoreset, uint64_t force_seed_step);
-int ssb_i_decima_obs(ssb_env *env, cudaStream_t s);  // the observation adapter kernel
-int ssb_i_decima_obs_cta(ssb_env *env, cudaStream_t s);  // its one-CTA-per-env version (ssb_policy.cu)
 // ssb_policy.cu
+int ssb_i_decima_obs(ssb_env *env, cudaStream_t s);  // the observation adapter kernel
 void ssb_i_policy_carve(Carver &cv, const ssb_config &c, const Dims &d, ssb::Params &p, uint32_t **pol_streams);
 int ssb_i_policy_init(ssb_env *env);
 void ssb_i_drop_decision_graph(ssb_env *env);

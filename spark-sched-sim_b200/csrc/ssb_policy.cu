@@ -14,8 +14,8 @@ namespace {
 // The observation adapter (DecimaObsWrapper.observation + make_dag_layer_edge_masks), one CTA per environment:
 // pass 1, one thread per active job: the job's edge count in the observation; an exclusive scan gives every job's
 // first edge entry (its first node row is the observation's dag_ptr); pass 2: the CTA's warps take the jobs
-// round-robin (Sim::decima_obs_job_w).  Same outputs as k_decima_obs (one warp per env, jobs one after the other),
-// which stays in the simulator's translation unit for the fused policy kernel and as the A/B reference.
+// round-robin (Sim::decima_obs_job_w).  Same outputs as Sim::decima_obs_w (one warp per env, jobs one after the
+// other), which the fused policy kernel runs.
 constexpr int ADAPTER_WARPS = 4;
 __global__ void __launch_bounds__(ADAPTER_WARPS * 32) k_decima_obs_cta(Params p)
 {
@@ -123,7 +123,6 @@ void ssb_i_policy_carve(Carver &cv, const ssb_config &c, const Dims &d, Params &
         p.pl_cnt = cv.take<int32_t>(tc::CNT_TOTAL);
         p.pl_ncand = cv.take<int32_t>(B);
         p.pl_bits = cv.take<unsigned long long>(B * d.Sc * 2);
-        p.pol_wblob = cv.take<float>(tc::BLOB_TOTAL);
         p.pol_wblob3 = cv.take<uint32_t>(fz::BLOB_TOTAL);
         p.pol_cand_rank = cv.take<int32_t>(B * d.Sc);
         p.fz_cursor = cv.take<int32_t>(4);
@@ -173,24 +172,18 @@ int launch_mlp_backward(int stage, ssb_env *env, const int32_t *list, const int3
                         const float *x_in = nullptr);
 template <int ST>
 int launch_tile(ssb_env *env, const int32_t *list, const int32_t *offset, const int32_t *count, int level,
-                int ctas_per_sm, cudaStream_t s, float *x_save = nullptr, size_t x_cap = 0)
+                cudaStream_t s, float *x_save = nullptr, size_t x_cap = 0)
 {
     tc::TileArgs a{list, offset, count, level};
     a.x_save = x_save;
     a.x_cap = (int)std::min<size_t>(x_cap, 0x7fffffff);
-    if (env->policy_mode == POLICY_TILES_TF32)
-        tc::k_tile_mlp<ST><<<env->num_sms * ctas_per_sm, 128, tc::Smem<ST>::BYTES, s>>>(env->p, a);
-    else
-        fz::k_tile3<ST><<<env->num_sms * (ctas_per_sm >= 4 ? fz::tile3_ctas<ST>() : ctas_per_sm), 128,
-                          sizeof(uint32_t) * fz::Blob<ST>::WORDS, s>>>(env->p, a);
+    fz::k_tile3<ST><<<env->num_sms * fz::tile3_ctas<ST>(), 128, sizeof(uint32_t) * fz::Blob<ST>::WORDS, s>>>(env->p, a);
     CUDA_TRY(cudaGetLastError());
     return SSB_OK;
 }
 template <int ST>
 int prepare_tile_kernel()
 {
-    CUDA_TRY(cudaFuncSetAttribute(tc::k_tile_mlp<ST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)tc::Smem<ST>::BYTES));
     CUDA_TRY(cudaFuncSetAttribute(fz::k_tile3<ST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)(sizeof(uint32_t) * fz::Blob<ST>::WORDS)));
     return SSB_OK;
@@ -205,7 +198,7 @@ int launch_mlp_backward(int stage, ssb_env *env, const int32_t *list, const int3
 }
 
 
-int ssb_i_decima_obs_cta(ssb_env *env, cudaStream_t s)
+int ssb_i_decima_obs(ssb_env *env, cudaStream_t s)
 {
     k_decima_obs_cta<<<env->p.B, ADAPTER_WARPS * 32, (sizeof(Sim::AdJob) + sizeof(int32_t)) * env->p.Jc, s>>>(env->p);
     CUDA_TRY(cudaGetLastError());
@@ -229,7 +222,10 @@ int ssb_i_policy_init(ssb_env *env)
     CUDA_TRY(cudaMemset(env->pol_streams, 0, sizeof(uint32_t) * (size_t)cfg->num_envs));  // stream 0 for every env
     {
         env->policy_mode = cfg->num_envs <= 2 * env->num_sms ? POLICY_FUSED : POLICY_TILES;
-        if (const char *pm = getenv("SSB_DECIMA_MODE")) env->policy_mode = std::max(0, std::min(atoi(pm), 2));
+        if (const char *pm = getenv("SSB_DECIMA_MODE")) {  // A/B override: 0 or 1; anything else keeps the default
+            if (!strcmp(pm, "0")) env->policy_mode = POLICY_TILES;
+            else if (!strcmp(pm, "1")) env->policy_mode = POLICY_FUSED;
+        }
         CUDA_TRY(cudaFuncSetAttribute(fz::fused::k_decima_fused, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)fz::fused::Smem::BYTES));
         {   // group size: one round of groups over the resident CTAs (two per SM) when that needs at most GMAX
@@ -281,16 +277,7 @@ int ssb_set_decima_weights(ssb_env *env, const float *weights, int32_t n_floats)
     }
     if (src != (size_t)dw::TOTAL || dst != (size_t)dd::TOTAL) return SSB_E_INVALID;
     CUDA_TRY(cudaMemcpy(env->p.pol_w, dev.data(), sizeof(float) * dd::TOTAL, cudaMemcpyHostToDevice));
-    // tensor-core path: per-stage blobs (canonical UMMA tiles, tf32 hi/lo halves, biases); padding stays zero
-    CUDA_TRY(cudaMemset(env->p.pol_wblob, 0, sizeof(float) * tc::BLOB_TOTAL));
-    tc::k_build_blob<tc::ST_PREP><<<1, 128>>>(env->p);
-    tc::k_build_blob<tc::ST_SINK><<<1, 128>>>(env->p);
-    tc::k_build_blob<tc::ST_MSG><<<1, 128>>>(env->p);
-    tc::k_build_blob<tc::ST_RCV><<<1, 128>>>(env->p);
-    tc::k_build_blob<tc::ST_DAG><<<1, 128>>>(env->p);
-    tc::k_build_blob<tc::ST_GLOB><<<1, 128>>>(env->p);
-    tc::k_build_blob<tc::ST_STAGE><<<1, 128>>>(env->p);
-    tc::k_build_blob<tc::ST_EXEC><<<1, 128>>>(env->p);
+    // tensor-core path: per-stage blobs (canonical UMMA tiles, bf16 three-term split, biases); padding stays zero
     CUDA_TRY(cudaMemset(env->p.pol_wblob3, 0, sizeof(uint32_t) * fz::BLOB_TOTAL));
     fz::k_build_blob<tc::ST_PREP><<<1, 128>>>(env->p.pol_w, env->p.pol_wblob3);
     fz::k_build_blob<tc::ST_SINK><<<1, 128>>>(env->p.pol_w, env->p.pol_wblob3);
@@ -362,8 +349,8 @@ static int decima_policy_impl(ssb_env *env, const int32_t *forced_stage, const i
     tc::k_pol_plan_scan<<<1, 32, 0, s>>>(p);
     tc::k_pol_plan_b<<<warp_grid, 128, 0, s>>>(p);
     CUDA_TRY(cudaGetLastError());
-    if ((rc = launch_tile<tc::ST_PREP>(env, p.pl_all, nullptr, cnt + tc::CNT_ALL, 0, 4, s))) return rc;
-    if ((rc = launch_tile<tc::ST_SINK>(env, p.pl_sink, nullptr, cnt + tc::CNT_SINK, 0, 4, s))) return rc;
+    if ((rc = launch_tile<tc::ST_PREP>(env, p.pl_all, nullptr, cnt + tc::CNT_ALL, 0, s))) return rc;
+    if ((rc = launch_tile<tc::ST_SINK>(env, p.pl_sink, nullptr, cnt + tc::CNT_SINK, 0, s))) return rc;
     // (an evaluation with the backward pass's scratch attached leaves every level's input rows there)
     float *xs = nullptr;
     size_t xcap = 0;
@@ -374,20 +361,18 @@ static int decima_policy_impl(ssb_env *env, const int32_t *forced_stage, const i
     }
     env->bw_saved = xs != nullptr;
     for (int k = env->dmax - 1; k >= 0; k--) {  // reversed(edge_masks) (scheduler.py:214-232)
-        if ((rc = launch_tile<tc::ST_MSG>(env, p.pl_lvl, cnt + tc::OFF_LVL + 2 * k, cnt + tc::CNT_LVL + 2 * k, k, 4, s, xs, xcap)))
+        if ((rc = launch_tile<tc::ST_MSG>(env, p.pl_lvl, cnt + tc::OFF_LVL + 2 * k, cnt + tc::CNT_LVL + 2 * k, k, s, xs, xcap)))
             return rc;
         if ((rc = launch_tile<tc::ST_RCV>(env, p.pl_lvl, cnt + tc::OFF_LVL + 2 * k + 1, cnt + tc::CNT_LVL + 2 * k + 1,
-                                          k, 4, s, xs, xcap)))
+                                          k, s, xs, xcap)))
             return rc;
     }
-    if ((rc = launch_tile<tc::ST_DAG>(env, p.pl_all, nullptr, cnt + tc::CNT_ALL, 0, 4, s))) return rc;
-    if ((rc = launch_tile<tc::ST_GLOB>(env, p.pl_jobs, nullptr, cnt + tc::CNT_JOBS, 0, 4, s))) return rc;
+    if ((rc = launch_tile<tc::ST_DAG>(env, p.pl_all, nullptr, cnt + tc::CNT_ALL, 0, s))) return rc;
+    if ((rc = launch_tile<tc::ST_GLOB>(env, p.pl_jobs, nullptr, cnt + tc::CNT_JOBS, 0, s))) return rc;
     tc::k_pol_glob_sum<<<(p.B + 7) / 8, 128, 0, s>>>(p);
-    // (score heads: four CTAs per SM in the TMEM path; round 1's shared-memory tiles fit one)
-    const int head_ctas = env->policy_mode == POLICY_TILES_TF32 ? 1 : 4;
-    if ((rc = launch_tile<tc::ST_STAGE>(env, nullptr, nullptr, cnt + tc::CNT_CAND, 0, head_ctas, s))) return rc;
+    if ((rc = launch_tile<tc::ST_STAGE>(env, nullptr, nullptr, cnt + tc::CNT_CAND, 0, s))) return rc;
     tc::k_pol_sample_stage<<<warp_grid, 128, 0, s>>>(p, forced_stage, env->pol_streams);
-    if ((rc = launch_tile<tc::ST_EXEC>(env, p.pl_exec, nullptr, cnt + tc::CNT_EXEC, 0, head_ctas, s))) return rc;
+    if ((rc = launch_tile<tc::ST_EXEC>(env, p.pl_exec, nullptr, cnt + tc::CNT_EXEC, 0, s))) return rc;
     tc::k_pol_sample_exec<<<warp_grid, 128, 0, s>>>(p, forced_num_exec, stage_idx_out, num_exec_out,
                                                     advance_draws ? 1 : 0, env->pol_streams);
     CUDA_TRY(cudaGetLastError());
@@ -673,14 +658,14 @@ int ssb_decima_backward(ssb_env *env, const float *grad_lgprob, const float *gra
         // the rows are already there when the evaluation this call differentiates ran with this scratch attached
         const bool have = env->bw_saved && env->bw_scratch == scratch && env->policy_mode != POLICY_FUSED;
         if (top > 0 && !have) {
-            if ((rc = launch_tile<tc::ST_PREP>(env, p.pl_all, nullptr, cnt + tc::CNT_ALL, 0, 4, s))) return rc;
-            if ((rc = launch_tile<tc::ST_SINK>(env, p.pl_sink, nullptr, cnt + tc::CNT_SINK, 0, 4, s))) return rc;
+            if ((rc = launch_tile<tc::ST_PREP>(env, p.pl_all, nullptr, cnt + tc::CNT_ALL, 0, s))) return rc;
+            if ((rc = launch_tile<tc::ST_SINK>(env, p.pl_sink, nullptr, cnt + tc::CNT_SINK, 0, s))) return rc;
         }
         for (int j = top - 1; j >= 0 && !have; j--) {
             const int32_t *om = cnt + tc::OFF_LVL + 2 * j, *cm = cnt + tc::CNT_LVL + 2 * j;
-            if ((rc = launch_tile<tc::ST_MSG>(env, p.pl_lvl, om, cm, j, 4, s, b.x_save, b.save_rows))) return rc;
+            if ((rc = launch_tile<tc::ST_MSG>(env, p.pl_lvl, om, cm, j, s, b.x_save, b.save_rows))) return rc;
             if (j > 0) {
-                if ((rc = launch_tile<tc::ST_RCV>(env, p.pl_lvl, om + 1, cm + 1, j, 4, s, b.x_save, b.save_rows))) return rc;
+                if ((rc = launch_tile<tc::ST_RCV>(env, p.pl_lvl, om + 1, cm + 1, j, s, b.x_save, b.save_rows))) return rc;
             } else {
                 CUDA_TRY(bwd::save_rows(tc::ST_RCV, p, env->num_sms, p.pl_lvl, om + 1, cm + 1, j, b.x_save, s));
             }
@@ -695,16 +680,16 @@ int ssb_decima_backward(ssb_env *env, const float *grad_lgprob, const float *gra
         }
     } else {
         for (int k = 0; k < top; k++) {
-            if ((rc = launch_tile<tc::ST_PREP>(env, p.pl_all, nullptr, cnt + tc::CNT_ALL, 0, 4, s))) return rc;
-            if ((rc = launch_tile<tc::ST_SINK>(env, p.pl_sink, nullptr, cnt + tc::CNT_SINK, 0, 4, s))) return rc;
+            if ((rc = launch_tile<tc::ST_PREP>(env, p.pl_all, nullptr, cnt + tc::CNT_ALL, 0, s))) return rc;
+            if ((rc = launch_tile<tc::ST_SINK>(env, p.pl_sink, nullptr, cnt + tc::CNT_SINK, 0, s))) return rc;
             for (int j = top - 1; j > k; j--) {
-                if ((rc = launch_tile<tc::ST_MSG>(env, p.pl_lvl, cnt + tc::OFF_LVL + 2 * j, cnt + tc::CNT_LVL + 2 * j, j, 4, s)))
+                if ((rc = launch_tile<tc::ST_MSG>(env, p.pl_lvl, cnt + tc::OFF_LVL + 2 * j, cnt + tc::CNT_LVL + 2 * j, j, s)))
                     return rc;
                 if ((rc = launch_tile<tc::ST_RCV>(env, p.pl_lvl, cnt + tc::OFF_LVL + 2 * j + 1,
-                                                  cnt + tc::CNT_LVL + 2 * j + 1, j, 4, s)))
+                                                  cnt + tc::CNT_LVL + 2 * j + 1, j, s)))
                     return rc;
             }
-            if ((rc = launch_tile<tc::ST_MSG>(env, p.pl_lvl, cnt + tc::OFF_LVL + 2 * k, cnt + tc::CNT_LVL + 2 * k, k, 4, s)))
+            if ((rc = launch_tile<tc::ST_MSG>(env, p.pl_lvl, cnt + tc::OFF_LVL + 2 * k, cnt + tc::CNT_LVL + 2 * k, k, s)))
                 return rc;
             if ((rc = launch_mlp_backward(tc::ST_RCV, env, p.pl_lvl, cnt + tc::OFF_LVL + 2 * k + 1,
                                           cnt + tc::CNT_LVL + 2 * k + 1, k, nullptr, gw, bw, s)))

@@ -184,7 +184,6 @@ struct Params {
     int32_t *pl_cnt;                               // counters, offsets, cursors (tc::CNT_*)
     int32_t *pl_ncand;                             // [B]
     unsigned long long *pl_bits;                   // [B * Sc][2] levels at which a node sends / receives
-    float *pol_wblob;  // per-stage weight blobs in shared-memory layout (tc::blob_offset)
     uint32_t *pol_wblob3;  // per-stage bf16 three-term weight blobs (fz::blob3_offset)
     int32_t *pol_cand_rank;  // [B][Sc] rank of a schedulable node among its env's schedulable nodes (its score's slot)
     int32_t *fz_cursor;      // [4] group cursor of the fused policy kernel

@@ -431,7 +431,7 @@ def test_full_backward_matches_torch_autograd(bank):
     """ssb_decima_backward(through_node_encoder=True): the gradients of all 42 tensors of the shipped model for
     loss = sum_b c1_b lgprob_b + c2_b entropy_b, against torch autograd through oracle/decima_torch.py (the whole
     policy over all envs in one batch: NodeEncoder with its level loop, DagEncoder, GlobalEncoder, both heads,
-    utils.evaluate) in float32.  Every tensor within 5e-4 of its largest entry (fp32 atomics; tf32x3 forward vs fp32)."""
+    utils.evaluate) in float32.  Every tensor within 5e-4 of its largest entry (fp32 atomics; bf16x3 forward vs fp32)."""
     import decima_torch
 
     from spark_sched_sim_b200.batched_env import BatchedSparkSchedSimEnv

@@ -7,14 +7,13 @@ accumulators and the shared tile matrix of k_mlp_backward carry over between til
 nine to sixty deep, and the batches mix envs that are live, finished, errored or empty.  Every execution path is
 compared: the list-driven tile kernels (mode 0) with the levels replayed by the backward pass, saved by the
 evaluation, or recomputed per level (SSB_BACKWARD_RECOMPUTE); the backward stopped above NodeEncoder (d loss / d h);
-the fused kernel (mode 1); round 1's tf32 shared-memory tiles (mode 2); a shuffled mini-batch gathered from stored
-observations with empty slots.
+the fused kernel (mode 1); a shuffled mini-batch gathered from stored observations with empty slots.
 
 Tolerance rule, for every compared quantity Q (scores, lgprob, entropy, each of the 42 gradient tensors, d_h):
     err_dev = max |Q_dev - Q_64|,  err_32 = max |Q_t32 - Q_64|   (Q_t32: the same restatement in float32, TF32 off)
     err_dev <= FP64_FACTOR * err_32 + C * max |Q_64|
 i.e. the device must be as close to fp64 as a straightforward float32 evaluation of the same batch, up to a small
-floor C relative to the quantity's own scale (float32 atomics over ~1e6 rows, bf16x3 / tf32x3 tensor-core products).
+floor C relative to the quantity's own scale (float32 atomics over ~1e6 rows, bf16x3 tensor-core products).
 For a gradient tensor max |Q_64| is taken over the six tensors of its MLP: a score head's last bias is a sum that
 cancels to ~0 (softmax is shift-invariant), and what remains of it on every side is the rounding of that MLP's terms."""
 import contextlib
@@ -31,10 +30,9 @@ pytestmark = pytest.mark.gpu
 
 FP64_FACTOR = 3.0
 # Measured on a B200 (1000 W), worst over the paths and shapes: err_dev / err_32 vs fp64 of
-#   scores   3.3e-5 / 9.7e-6 of 17.8 (mode 2; modes 0 / 1: 1.5e-5 / 9.2e-6 of 10.2)
-#   lgprob   1.1e-5 / 2.7e-6 of 8.0  (mode 2; modes 0 / 1: 5.4e-6 / 2.6e-6)
-#   entropy  1.8e-6 / 2.6e-7 of 0.68 (mode 2, the only path that needs the floor: round 1's tiles split every operand
-#            into two tf32 halves, 22 of float32's 24 bits; modes 0 / 1: 3.6e-7 / 2.6e-7)
+#   scores   1.5e-5 / 9.2e-6 of 10.2
+#   lgprob   5.4e-6 / 2.6e-6
+#   entropy  3.6e-7 / 2.6e-7
 #   grad     7.7e-4 / 3.0e-5 of 57.5 (the job summary's MLP at the wide shape, every path alike: float32 sums over
 #            1.7e5 rows in per-CTA registers and atomics, torch's in a reduction tree)
 #   d_h      2.1e-6 / 3.6e-7 of 1.6
@@ -201,21 +199,21 @@ def test_evaluate_and_backward_at_training_sizes_against_fp64(shape, monkeypatch
     c2 = torch.randn(B, device="cuda", generator=g)
     check = _Check()
     print(f"\n{shape}: {B} envs, {E} executors, {torch.cuda.get_device_name(0)}")
-    for mode, paths in (("0", ("replay", "to-h", "saved", "recompute")), ("1", ("fused",)), ("2", ("tf32-saved",))):
+    for mode, paths in (("0", ("replay", "to-h", "saved", "recompute")), ("1", ("fused",))):
         env = _make_env(shape, mode, monkeypatch)
         snap = env.decima_snapshot()
         env.decima_policy()
         act, lg_sampled = env.pol_action.clone(), env.pol_lgprob.clone()
         refs = {}
         for path in paths:  # ("replay" first: once a backward has attached its scratch, evaluations save the levels)
-            out = _evaluate(env, snap, act, for_backward=path in ("saved", "tf32-saved"), c1=c1, c2=c2,
+            out = _evaluate(env, snap, act, for_backward=path == "saved", c1=c1, c2=c2,
                             through=path != "to-h", recompute=path == "recompute", monkeypatch=monkeypatch)
             assert torch.equal(out["obs"]["action"][:, [0, 2]], act[:, [0, 2]]), (shape, path)
             assert torch.equal(out["lgprob"], lg_sampled), (shape, path, "evaluate's lgprob != the sampled one")
             key = path == "to-h"
             if key not in refs:
                 refs[key] = _reference(out["obs"], c1, c2, E, to_h=key)
-            if path in ("replay", "fused", "tf32-saved"):
+            if path in ("replay", "fused"):
                 obs = out["obs"]
                 live = obs["live"]
                 depth = int(obs["depth"][live].max()) if live.any() else 0

@@ -15,7 +15,7 @@ pytestmark = pytest.mark.gpu
 
 CFG = {"num_executors": 10, "job_arrival_cap": 4, "job_arrival_rate": 4.0e-5, "moving_delay": 2000.0,
        "warmup_delay": 1000.0}
-MODES = {"tiles": "0", "fused": "1", "tf32": "2"}
+MODES = {"tiles": "0", "fused": "1"}
 
 
 def _weights():
