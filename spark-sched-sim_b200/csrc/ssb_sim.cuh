@@ -529,13 +529,6 @@ struct Sim {
         if (lane == 0) { h->n_sched = total; stats->sched_scans++; }
         return total;
     }
-    __device__ void clear_sched_w()
-    {
-        int n_active = h->n_active;
-        for (int i = lane; i < n_active; i += 32) jb[act[i]].sched = 0;
-        if (lane == 0) h->n_sched = 0;
-        __syncwarp();
-    }
     // first schedulable stage of the job-id list semantics used by _find_backup_stage (:821-845)
     __device__ bool first_schedulable(bool only_job, int job, int source_job_arg, int &oj, int &os)
     {
@@ -720,6 +713,8 @@ struct Sim {
     {
         act[h->n_active++] = (int16_t)j;
         jb[j].state = JOB_ACTIVE;
+        h->n_obs_nodes += jb[j].n_stages;  // every stage and template edge of a new job is in the observation
+        h->n_obs_edges += jb[j].n_obs_edges;
         if (pool_size(POOL_COMMON) > 0) h->source = POOL_COMMON;
     }
     __device__ void handle_executor_arrival(int e, int j, int s)  // :440-450
@@ -739,6 +734,13 @@ struct Sim {
     {
         JobRec &J = jb[j];
         J.active &= ~bit64(s);
+        {   // the observation loses node s and its job's edges to it or from it (a completed job has none left, so
+            // process_job_completion has nothing to subtract)
+            const int eb = p.b_edge_base[J.tmpl], m = job_obs_edges(J.active, eb, p.b_edge_base[J.tmpl + 1] - eb);
+            h->n_obs_nodes -= 1;
+            h->n_obs_edges += m - J.n_obs_edges;
+            J.n_obs_edges = (int16_t)m;
+        }
         SSB_CHKR(J.frontier & bit64(s), false);
         J.frontier &= ~bit64(s);
         uint64_t kids = p.b_child[J.ts_base + s] & J.active, fresh = 0;
@@ -1506,7 +1508,7 @@ struct Sim {
 
     // ------------------------------------------------------------ _observe (:345-406, utils.py:5-22)
     // edges of a job's template (ne entries from eb) with both ends active: the job's edges in the observation
-    // (utils.subgraph, utils.py:5-22); one thread per job
+    // (utils.subgraph, utils.py:5-22); one thread per job (lane 0 at a stage completion)
     __device__ int job_obs_edges(uint64_t active, int eb, int ne) const
     {
         int c = 0;
@@ -1518,8 +1520,9 @@ struct Sim {
         return c;
     }
     // What observe_w writes: OBS_FULL = header, observation counters and the graph slabs (dag_ptr, exec_supplies,
-    // nodes, edge_links).  The fused rollout splits it: OBS_HDR every decision (the header and the counters, from
-    // a count pass with one lane per active job), OBS_GRAPH once when its decision loop ends (the slabs only).
+    // nodes, edge_links).  The fused rollout splits it: OBS_HDR every decision (the header and the counters, with
+    // the node and edge counts the simulator keeps in EnvHdr), OBS_GRAPH once when its decision loop ends (the slabs
+    // only).  OBS_FULL counts the graph it writes, independently of the kept counts.
     enum : int { OBS_HDR = 1, OBS_GRAPH = 2, OBS_FULL = OBS_HDR | OBS_GRAPH };
     template <int PARTS = OBS_FULL>
     __device__ SSB_COLD void observe_w(double reward, bool terminated)
@@ -1532,22 +1535,13 @@ struct Sim {
         const int src_job = source_job_id();
         int src_idx = n_active, N = 0, M = 0;
         if constexpr (PARTS == OBS_HDR) {
-            for (int base = 0; base < n_active; base += 32) {
+            N = h->n_obs_nodes;
+            M = h->n_obs_edges;
+            for (int base = 0; base < n_active && src_job >= 0; base += 32) {
                 const int i = base + lane;
-                int j = -1;
-                if (i < n_active) {
-                    j = act[i];
-                    const JobRec &J = jb[j];
-                    const uint64_t active = J.active;
-                    const int eb = p.b_edge_base[J.tmpl];
-                    N += popc64(active);
-                    M += job_obs_edges(active, eb, p.b_edge_base[J.tmpl + 1] - eb);
-                }
-                unsigned hit = __ballot_sync(FULL, j >= 0 && j == src_job);
-                if (hit) src_idx = base + __ffs(hit) - 1;
+                const unsigned hit = __ballot_sync(FULL, i < n_active && act[i] == src_job);
+                if (hit) { src_idx = base + __ffs(hit) - 1; break; }
             }
-            N = __reduce_add_sync(FULL, N);
-            M = __reduce_add_sync(FULL, M);
         } else {
             // dag_ptr / exec_supplies / source_job_idx: exclusive scan of per-job active-stage counts
             for (int base = 0; base < n_active; base += 32) {
@@ -1701,21 +1695,25 @@ struct Sim {
         }
         // commitment round has completed (:195-199)
         const int n_active0 = h->n_active;
-        for (int i = lane; i < n_active0; i += 32) p.old_act[(size_t)b * p.Jc + i] = act[i];
-        __syncwarp();
         if (lane == 0) {
             commit_remaining_executors();
             fulfill_commitments_from_source();
             h->source = POOL_NONE;
             h->wall_old = h->wall_time;
             h->n_old_active = n_active0;
+            h->n_sched = 0;
         }
         __syncwarp();
-        // selected_stages.clear() comes AFTER the fulfilment: backup scheduling during it must
-        // still see this round's selections (:197-199, :825-839)
-        for (int i = lane; i < n_active0; i += 32) jb[act[i]].selected = 0;
+        // one pass over the active jobs (no job arrives or completes during the fulfilment): the reward's copy of the
+        // active list, selected_stages.clear() -- AFTER the fulfilment, whose backup scheduling must still see this
+        // round's selections (:197-199, :825-839) -- and the schedulable stages cleared
+        for (int i = lane; i < n_active0; i += 32) {
+            const int j = act[i];
+            p.old_act[(size_t)b * p.Jc + i] = (int16_t)j;
+            jb[j].selected = 0;
+            jb[j].sched = 0;
+        }
         __syncwarp();
-        clear_sched_w();
         SSB_TACC(5);
         return 1;
     }
@@ -1859,6 +1857,7 @@ struct Sim {
             H.policy_draws = 0;
             H.hist_n = 0;
             H.obs_owed = 0;
+            H.n_obs_nodes = 0; H.n_obs_edges = 0;  // (the arrivals below add their jobs)
         }
         __syncwarp();
         if (h->error) {
@@ -1883,6 +1882,7 @@ struct Sim {
             for (int s = 0; s < ns; s++)
                 if (p.b_parent[J.ts_base + s] == 0) fr |= bit64(s);  // job.py:93-111 in-degree 0
             J.frontier = fr;
+            J.n_obs_edges = (int16_t)(p.b_edge_base[t + 1] - p.b_edge_base[t]);
             J.sat = 0; J.sched = 0; J.selected = 0;
             J.n_local = 0; J.supply = 0; J.commit_from = 0; J.sat_count = 0; J.state = JOB_PENDING;
         }

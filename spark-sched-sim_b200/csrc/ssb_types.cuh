@@ -68,7 +68,8 @@ struct __align__(16) JobRec {  // job.py:12-40 + tracker counters keyed by the j
     int16_t commit_from;  // _num_commitments_from[(job, None)]
     uint8_t sat_count;    // saturated_stage_count
     uint8_t state;
-    uint8_t pad[6];
+    int16_t n_obs_edges;  // template edges with both ends in `active`: the job's edges in the observation
+    uint8_t pad[4];
 };
 static_assert(sizeof(JobRec) == 96, "JobRec layout");
 
@@ -110,8 +111,11 @@ struct __align__(16) EnvHdr {
     uint32_t policy_draws;  // Philox policy-stream counter (on-device action sampling)
     int32_t hist_n;         // add_history calls of this episode (rows beyond hist_cap are counted, not stored)
     int32_t obs_owed;  // k_rollout_fair: parts of the live observation still to be written (Sim::OWE_*), 0 outside it
-    int32_t pad2;
+    // nodes and edges of the observation (active stages of the active jobs, edges between them), kept current where
+    // a job's `active` or the active-job list changes, so that the per-decision observation header needs no count pass
+    int32_t n_obs_nodes, n_obs_edges;
 };
+static_assert(sizeof(EnvHdr) == 160, "EnvHdr layout");
 
 // Everything a kernel needs, passed by value.
 struct Params {
