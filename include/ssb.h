@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define SSB_ABI_VERSION 9
+#define SSB_ABI_VERSION 10
 
 /* status codes of the entry points */
 enum {
@@ -478,11 +478,64 @@ int ssb_rollout_decima_async(ssb_env *env, int32_t max_decisions, double rollout
  * snapshot is loaded (ssb_decima_snapshot_load) and on a handle without the policy. */
 int ssb_decima_attach_rollout_store(ssb_env *env, void *snapshots, int32_t capacity, int32_t *stage_sel,
                                     int32_t *exec_sel);
+/* Episode statistics that survive resets (RecordEpisodeStatistics for the batched env, and the reference's
+ * job_duration_buff, spark_sched_sim.py:83, :243-245, :697).  The caller owns the memory, all DEVICE:
+ *   episodes      ssb_episode[B][capacity]: a ring of finished episodes per env, or NULL with capacity 0
+ *   job_durations f64[B][window]: a ring of completed-job durations (ms) per env, or NULL with window 0
+ *   cursors       ssb_episode_cursor[B]; NULL detaches (nothing is written from then on)
+ * What is recorded:
+ *   - One record per episode, for the step whose observation first reports terminated or truncated
+ *     (wall_time >= time_limit, the test of the observation header), written by the call that ran that step (before
+ *     any reset that follows it): ssb_step (eager and budgeted), the *_host steps, the fused fair / FIFO / random
+ *     rollouts (sync and async) and the Decima rollouts.  Env b's record k goes to
+ *     episodes[b][k % capacity]; cursors[b].episodes counts the records.  A truncated env that is stepped again writes
+ *     no second record.  No record is written for an episode abandoned by an explicit ssb_reset / ssb_reset_host, an
+ *     env frozen by an invariant error (ssb_obs_hdr.error >= 1000), or a reset refused with SSB_ENV_CAPACITY /
+ *     SSB_ENV_NO_LIMIT.  An episode that is live when the log is attached counts its decisions from the attach.
+ *   - job_time and sum_job_duration are summed serially in job-index order (f64, no contraction), so a host loop
+ *     over the jobs restates them bit for bit.
+ *   - Every job completion (spark_sched_sim.py:697 appends it there) puts t_completed - t_arrival at
+ *     job_durations[b][n % window], n = cursors[b].jobs_completed before the completion, in completion-time order
+ *     (job index among equal times: the order of the facade's host deque, env.py; the reference appends in event
+ *     order, so two jobs that complete at the same wall time may stand in the other order than there).  The
+ *     window and jobs_completed are brought up to date by every call that steps the envs, before it returns (and
+ *     inside the fused rollouts before each in-kernel reset).  Resets do
+ *     not touch the window, as in the reference: completions of episodes that were later abandoned count too.
+ * Attaching fills the library-use fields of the cursors from the live state (stream-ordered on `stream`) and leaves
+ * episodes / jobs_completed as given: zero them for a fresh log, keep them to continue one (e.g. on a re-created
+ * handle).  The rings are not read by the library except for ssb_collect_stats [6..7].  ssb_reset_stats keeps the
+ * decision count of a live episode right.  Refused (SSB_E_INVALID): capacity or window < 0, a NULL ring with a
+ * positive size or a ring with size 0. */
+typedef struct {              /* one finished episode, 64 B */
+    uint64_t seed;            /* the episode's seed */
+    double wall_time;         /* wall time of the observation that ended it (ms) */
+    double time_limit;        /* the episode's limit (+inf if none) */
+    double job_time;          /* sum over arrived jobs of min(t_completed, wall_time) - t_arrival (job-ms):
+                                 metrics.avg_num_jobs * wall_time, and minus the undiscounted episode return when
+                                 beta = 0 (up to rounding) */
+    double sum_job_duration;  /* sum over completed jobs of t_completed - t_arrival (ms) */
+    int32_t decisions;        /* step() calls accepted in the episode (ssb_stats.decisions counting) */
+    int32_t jobs_arrived, jobs_completed;
+    int32_t flags;            /* 1 terminated, 2 truncated */
+    int32_t episode;          /* index of the episode since the env's last ssb_reset (0 = the one ssb_reset started) */
+    int32_t pad;
+} ssb_episode;
+typedef struct {              /* per env, 32 B */
+    int64_t episodes;         /* episodes recorded since the counts were zeroed; slot = episodes % capacity */
+    int64_t jobs_completed;   /* completions recorded; slot = jobs_completed % window */
+    uint64_t decisions0;      /* library use: ssb_stats.decisions at the live episode's start */
+    int32_t ended;            /* library use: the live episode has been recorded */
+    int32_t logged;           /* library use: completions of the live episode already in the window */
+} ssb_episode_cursor;
+int ssb_attach_episode_log(ssb_env *env, ssb_episode *episodes, int32_t capacity, double *job_durations,
+                           int32_t window, ssb_episode_cursor *cursors, void *stream);
 /* collect_stats (trainers/rollout_worker.py:122-129) over all envs as SUMS that can be all-reduced across GPUs:
  * out = DEVICE f64[8]: [0] sum over envs of avg_num_jobs = (total job time so far) / wall_time
  * (metrics.py:15-16; envs at wall_time 0 skipped), [1] number of envs counted in [0], [2] completed jobs,
- * [3] job arrivals (completed + active), [4] sum of the completed jobs' durations in ms (current episodes; the
- * reference's avg_job_duration averages its last 200 completions across resets), [5] sum of wall times, [6..7] 0.
+ * [3] job arrivals (completed + active), [4] sum of the completed jobs' durations in ms (current episodes only),
+ * [5] sum of wall times, [6] with an episode log that has a job-duration window: sum over the envs with at least one
+ * stored duration of the mean of that env's stored durations (ms) -- the reference's env.avg_job_duration, the mean
+ * of its last `window` completions across resets -- and [7] the number of such envs; 0 and 0 otherwise.
  * Fixed summation order (deterministic). */
 int ssb_collect_stats(ssb_env *env, double *out, void *stream);
 /* device pointer to ssb_stats[B] */

@@ -9,7 +9,7 @@ import numpy as np
 
 PKG_DIR = osp.dirname(osp.abspath(__file__))
 LIB_PATH = osp.join(PKG_DIR, "_lib", "libssb.so")
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 
 class SsbConfig(C.Structure):
@@ -136,11 +136,19 @@ assert TRANSITION_DTYPE.itemsize == 32
 STATS_FIELDS = ("decisions", "events", "sched_scans", "sum_nodes", "sum_edges", "sum_jobs",
                 "observations", "episodes")
 STATS_DTYPE = np.dtype([(f, "<u8") for f in STATS_FIELDS])
+# ssb_episode / ssb_episode_cursor (include/ssb.h): the episode log of ssb_attach_episode_log
+EPISODE_DTYPE = np.dtype([("seed", "<u8"), ("wall_time", "<f8"), ("time_limit", "<f8"), ("job_time", "<f8"),
+                          ("sum_job_duration", "<f8"), ("decisions", "<i4"), ("jobs_arrived", "<i4"),
+                          ("jobs_completed", "<i4"), ("flags", "<i4"), ("episode", "<i4"), ("pad", "<i4")])
+assert EPISODE_DTYPE.itemsize == 64
+EPISODE_CURSOR_DTYPE = np.dtype([("episodes", "<i8"), ("jobs_completed", "<i8"), ("decisions0", "<u8"),
+                                 ("ended", "<i4"), ("logged", "<i4")])
+assert EPISODE_CURSOR_DTYPE.itemsize == 32
 
 EXPORTS = [
     "ssb_abi_version", "ssb_last_cuda_error", "ssb_workspace_bytes", "ssb_create", "ssb_destroy",
     "ssb_load_trace", "ssb_clear_trace", "ssb_reset", "ssb_step", "ssb_reset_host", "ssb_step_host", "ssb_step_fair_host", "ssb_set_autoreset", "ssb_set_mean_time_limit",
-    "ssb_rollout_fair", "ssb_rollout_fair_traj", "ssb_rollout_fair_async", "ssb_discounted_returns", "ssb_differential_returns", "ssb_group_baselines", "ssb_ppo_loss", "ssb_adam_step", "ssb_fair_actions", "ssb_random_actions", "ssb_rollout_random", "ssb_rollout_random_async", "ssb_get_views", "ssb_get_stats", "ssb_collect_stats", "ssb_reset_stats",
+    "ssb_rollout_fair", "ssb_rollout_fair_traj", "ssb_rollout_fair_async", "ssb_discounted_returns", "ssb_differential_returns", "ssb_group_baselines", "ssb_ppo_loss", "ssb_adam_step", "ssb_fair_actions", "ssb_random_actions", "ssb_rollout_random", "ssb_rollout_random_async", "ssb_get_views", "ssb_get_stats", "ssb_collect_stats", "ssb_reset_stats", "ssb_attach_episode_log",
     "ssb_get_jobs", "ssb_get_log", "ssb_get_history", "ssb_decima_obs", "ssb_get_decima_views",
     "ssb_set_decima_weights", "ssb_decima_policy", "ssb_rollout_decima", "ssb_rollout_decima_async", "ssb_set_policy_streams", "ssb_decima_attach_rollout_store", "ssb_decima_snapshot_bytes",
     "ssb_decima_snapshot", "ssb_decima_snapshot_gather", "ssb_decima_snapshot_load", "ssb_decima_snapshot_unload", "ssb_decima_evaluate", "ssb_decima_head_adjoint", "ssb_decima_head_backward", "ssb_decima_backward_bytes", "ssb_decima_attach_backward_scratch", "ssb_decima_backward", "ssb_get_policy_views", "ssb_decima_work", "ssb_decima_mlp_rows", "ssb_packed_obs_bytes", "ssb_get_obs_host", "ssb_get_debug_counters",
@@ -219,6 +227,7 @@ def lib():
     L.ssb_get_stats.argtypes = [vp, C.POINTER(vp)]
     L.ssb_reset_stats.argtypes = [vp, vp]
     L.ssb_collect_stats.argtypes = [vp, vp, vp]
+    L.ssb_attach_episode_log.argtypes = [vp, vp, i32, vp, i32, vp, vp]
     L.ssb_get_debug_counters.argtypes = [vp, C.POINTER(vp)]
     L.ssb_get_jobs.argtypes = [vp, i32, C.POINTER(i32), vp, vp, vp, vp, i32]
     L.ssb_get_log.argtypes = [vp, i32, i64, i64, C.POINTER(i64)] + [vp] * 7

@@ -134,8 +134,8 @@ class BatchedSparkSchedSimEnv:
     def grow(self, max_jobs: int) -> None:
         """Re-creates the handle with room for `max_jobs` jobs per env (node / edge / pool capacities follow).  The
         capacity is fixed at creation (one workspace, carved once), so growing means a new handle: every env's
-        state is lost (reset afterwards); the policy weights, the policy sampling streams, the auto-reset mode and the
-        mean time limit are carried over.  Time-limited arrivals without a job cap are the case that needs this: an episode that draws
+        state is lost (reset afterwards); the policy weights, the policy sampling streams, the auto-reset mode,
+        the mean time limit and the episode log (attach_episode_log) are carried over.  Time-limited arrivals without a job cap are the case that needs this: an episode that draws
         more jobs than the capacity stops at its reset with SSB_ENV_CAPACITY (`reset_host(..., grow=True)` grows
         and retries; `required_job_capacity` sizes the handle up front)."""
         assert max_jobs > self.max_jobs
@@ -150,6 +150,8 @@ class BatchedSparkSchedSimEnv:
             self.set_mean_time_limit(self._settings["mean_time_limit"])
         if "policy_streams" in self._settings:
             self.set_policy_streams(self._settings["policy_streams"])
+        if "episode_log" in self._settings:
+            self._attach_episode_log()  # the same buffers: the records, counts and window carry over
 
     @staticmethod
     def required_job_capacity(job_arrival_rate: float, mean_time_limit: float, tail: float = 1e-9) -> int:
@@ -419,6 +421,89 @@ class BatchedSparkSchedSimEnv:
 
     def reset_stats(self):
         nat.check(self.L.ssb_reset_stats(self._h, self._stream()), "ssb_reset_stats")
+
+    # ---------------------------------------------------------------- episode log (ssb_attach_episode_log)
+    def attach_episode_log(self, capacity: int = 64, window: int = 200) -> None:
+        """Records every finished episode on the device -- a RecordEpisodeStatistics for the batched env -- in a
+        ring of `capacity` records per env, and every completed job's duration in a ring of the last `window` per env
+        (the reference's job_duration_buff, deque(maxlen=200), which survives resets).  The three buffers are device
+        tensors of this object, zeroed here; grow() re-attaches the same ones, so the log and the window carry over.
+        Read them with episodes() and job_duration_window(); collect_stats()[6:8] then carries the window's means."""
+        B, cap, win = self.num_envs, int(capacity), int(window)
+        if cap < 0 or win < 0:
+            raise ValueError("capacity and window must be >= 0")
+        rec = torch.zeros(max(B * cap * nat.EPISODE_DTYPE.itemsize, 1), dtype=torch.uint8, device=self.device)
+        dur = torch.zeros(B, max(win, 1), dtype=torch.float64, device=self.device)
+        cur = torch.zeros(B * nat.EPISODE_CURSOR_DTYPE.itemsize, dtype=torch.uint8, device=self.device)
+        self._settings["episode_log"] = (rec, cap, dur, win, cur)
+        self._attach_episode_log()
+
+    def _attach_episode_log(self) -> None:
+        rec, cap, dur, win, cur = self._settings["episode_log"]
+        nat.check(self.L.ssb_attach_episode_log(self._h, rec.data_ptr() if cap else None, cap,
+                                                dur.data_ptr() if win else None, win, cur.data_ptr(), self._stream()),
+                  "ssb_attach_episode_log")
+
+    def detach_episode_log(self) -> None:
+        """Stops recording; the buffers are released."""
+        nat.check(self.L.ssb_attach_episode_log(self._h, None, 0, None, 0, None, self._stream()),
+                  "ssb_attach_episode_log")
+        self._settings.pop("episode_log", None)
+
+    def _episode_log(self):
+        if "episode_log" not in self._settings:
+            raise RuntimeError("no episode log attached (attach_episode_log())")
+        return self._settings["episode_log"]
+
+    def episode_cursors(self) -> torch.Tensor:
+        """The per-env cursors as an int64 device tensor [B, 4]: episodes recorded, jobs completed, and the two
+        library-use words."""
+        return self._episode_log()[4].view(torch.int64).view(self.num_envs, 4)
+
+    def episodes(self) -> dict:
+        """The stored episode records, flattened env-major and oldest first within an env, as device tensors:
+        env, seed (int64 holding the u64 seed), wall_time, time_limit, job_time, sum_job_duration (f64), decisions,
+        jobs_arrived, jobs_completed, flags, episode (i32), terminated / truncated (bool), avg_job_duration (seconds,
+        sum_job_duration / jobs_completed * 1e-3, nan without a completed job), avg_num_jobs (job_time / wall_time),
+        and dropped: per env [B], the records the ring has overwritten.  Synchronises (the count is data-dependent)."""
+        rec, cap, _, _, _ = self._episode_log()
+        B = self.num_envs
+        n_rec = self.episode_cursors()[:, 0]
+        stored = n_rec.clamp(max=cap)
+        k = torch.arange(max(cap, 1), device=self.device)
+        env, kk = (k[None, :] < stored[:, None]).nonzero(as_tuple=True)
+        slot = (n_rec[env] - stored[env] + kk) % max(cap, 1)
+        rows = rec[:B * cap * nat.EPISODE_DTYPE.itemsize].view(torch.int64).view(B, max(cap, 1) if cap else 0, 8)
+        r = rows[env, slot] if cap else torch.zeros(0, 8, dtype=torch.int64, device=self.device)
+        f, i = r.view(torch.float64), r.view(torch.int32)
+        jc = i[:, 12]
+        out = {"env": env.to(torch.int32), "seed": r[:, 0], "wall_time": f[:, 1], "time_limit": f[:, 2],
+               "job_time": f[:, 3], "sum_job_duration": f[:, 4], "decisions": i[:, 10], "jobs_arrived": i[:, 11],
+               "jobs_completed": jc, "flags": i[:, 13], "episode": i[:, 14]}
+        out["terminated"] = (out["flags"] & 1) != 0
+        out["truncated"] = (out["flags"] & 2) != 0
+        out["avg_job_duration"] = torch.where(jc > 0, out["sum_job_duration"] / jc.clamp(min=1) * 1e-3,
+                                              torch.full_like(out["sum_job_duration"], float("nan")))
+        out["avg_num_jobs"] = out["job_time"] / out["wall_time"]
+        out["dropped"] = n_rec - stored
+        return out
+
+    def clear_episodes(self) -> None:
+        """Zeroes every env's episode count (stream-ordered); the job-duration window is left as it is."""
+        self.episode_cursors()[:, 0].zero_()
+
+    def job_duration_window(self) -> tuple[torch.Tensor, torch.Tensor]:
+        """(durations f64 [B, window] in ms, oldest to newest, nan past the fill; fill i64 [B]): env b's last
+        min(completions, window) completed-job durations, across resets."""
+        _, _, dur, win, _ = self._episode_log()
+        n = self.episode_cursors()[:, 1]
+        if win == 0:
+            return torch.zeros(self.num_envs, 0, dtype=torch.float64, device=self.device), torch.zeros_like(n)
+        fill = n.clamp(max=win)
+        k = torch.arange(win, device=self.device)
+        idx = (n[:, None] - fill[:, None] + k[None, :]) % win
+        vals = dur.gather(1, idx)
+        return torch.where(k[None, :] < fill[:, None], vals, torch.full_like(vals, float("nan"))), fill
 
     def obs(self, b: int = 0, hdr: np.ndarray | None = None) -> dict:
         """Observation of environment b as host arrays (the pieces of the reference obs dict)."""

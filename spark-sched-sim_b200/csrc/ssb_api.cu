@@ -112,14 +112,23 @@ k_rollout_fair_async(Params p, int max_decisions, double duration, int dynamic_p
 }
 
 // collect_stats sums in a fixed order: block k reduces the envs k, k + STATS_BLOCKS, ... (one warp per env, lanes
-// over its jobs) into part[k][6]; a last warp adds the blocks' partial sums in block order.
-constexpr int STATS_BLOCKS = 128;
+// over its jobs) into part[k][8]; a last warp adds the blocks' partial sums in block order.
 __global__ void __launch_bounds__(256) k_collect_stats_part(Params p, double *part)
 {
-    __shared__ double sh[8][6];
+    __shared__ double sh[8][8];
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    double acc[6] = {0, 0, 0, 0, 0, 0};
+    double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    const EpisodeLog *L = episode_log(p);
+    const int W = L->cur ? L->window : 0;
     for (int b = (int)blockIdx.x + w * STATS_BLOCKS; b < p.B; b += 8 * STATS_BLOCKS) {
+        if (W > 0) {  // the mean of the env's stored job durations (the reference's avg_job_duration, in ms)
+            const long long nc = L->cur[b].jobs_completed;
+            const int n = nc < W ? (int)nc : W;
+            double s = 0.0;
+            for (int i = lane; i < n; i += 32) s += L->win[(size_t)b * W + i];
+            for (int off = 16; off; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
+            if (n > 0) { acc[6] += s / n; acc[7] += 1.0; }
+        }
         const EnvHdr &h = p.hdr[b];
         const JobRec *jb = p.job + (size_t)b * p.Jc;
         const double wall = h.wall_time;
@@ -141,9 +150,9 @@ __global__ void __launch_bounds__(256) k_collect_stats_part(Params p, double *pa
         acc[2] += nc; acc[3] += na; acc[4] += cd; acc[5] += wall;
     }
     if (lane == 0)
-        for (int i = 0; i < 6; i++) sh[w][i] = acc[i];
+        for (int i = 0; i < 8; i++) sh[w][i] = acc[i];
     __syncthreads();
-    if (threadIdx.x < 6) {
+    if (threadIdx.x < 8) {
         double s = 0.0;
         for (int i = 0; i < 8; i++) s += sh[i][threadIdx.x];
         part[(size_t)blockIdx.x * 8 + threadIdx.x] = s;
@@ -153,10 +162,35 @@ __global__ void k_collect_stats_final(const double *part, double *out)
 {
     if (threadIdx.x < 8) {
         double s = 0.0;
-        if (threadIdx.x < 6)
-            for (int k = 0; k < STATS_BLOCKS; k++) s += part[(size_t)k * 8 + threadIdx.x];
+        for (int k = 0; k < STATS_BLOCKS; k++) s += part[(size_t)k * 8 + threadIdx.x];
         out[threadIdx.x] = s;
     }
+}
+
+// ssb_attach_episode_log: after every launch that steps the envs (only while a log is attached), the records of the
+// episodes that launch ended and the job completions it made (Sim::log_launch_w)
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32) k_episode_log(Params p)
+{
+    const int b = blockIdx.x * WARPS_PER_CTA + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (b >= p.B) return;
+    Sim sim(p, b, lane);
+    sim.log_launch_w();
+}
+
+// ssb_attach_episode_log: publishes the descriptor (L.cur == nullptr: detached) and fills every env's library-use
+// cursor fields from its live state (the counts are the caller's)
+__global__ void k_attach_episode_log(Params p, EpisodeLog L)
+{
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b == 0) *episode_log(p) = L;
+    if (b >= p.B || !L.cur) return;
+    const EnvHdr &h = p.hdr[b];
+    ssb_episode_cursor &c = L.cur[b];
+    c.decisions0 = p.stats[b].decisions;
+    c.ended = (h.error || h.done || h.wall_time >= h.time_limit) ? 1 : 0;  // nothing live to record
+    c.logged = h.n_completed;  // the window starts with the completions after the attach
+    JobRec *jb = p.job + (size_t)b * p.Jc;
+    for (int j = 0; j < h.next_arrival; j++) jb[j].logged = jb[j].state == JOB_COMPLETED;
 }
 
 // ---- packed observations: the rows of every env's observation back to back (what a host caller copies out)
@@ -203,10 +237,14 @@ k_pack_copy(Params p, const int32_t *offsets, float *nodes, int32_t *edges, int3
     for (int i = lane; i < o.num_active_jobs; i += 32) supplies[oj + i] = p.obs_supplies[(size_t)b * p.Jc + i];
 }
 
-__global__ void k_zero_stats(ssb_stats *s, int n)
+// cur (the attached episode log's cursors, may be nullptr): decisions0 moves with the counter, modulo 2^64, so that a
+// live episode's decision count stays what it was
+__global__ void k_zero_stats(ssb_stats *s, int n, ssb_episode_cursor *cur)
 {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) s[i] = ssb_stats{};
+    if (i >= n) return;
+    if (cur) cur[i].decisions0 -= s[i].decisions;
+    s[i] = ssb_stats{};
 }
 
 // ------------------------------------------------------------------------------------ workspace
@@ -272,7 +310,7 @@ void carve(Carver &cv, const ssb_config &c, const ssb_bank &bk, const Dims &d, P
     p.log = cv.take<LogRow>(c.log_capacity > 0 ? B * (size_t)c.log_capacity : 1);
     p.hist = cv.take<HistRow>(c.history_capacity > 0 ? B * (size_t)c.history_capacity : 1);
     p.stats = cv.take<ssb_stats>(B);
-    p.stats_part = cv.take<double>(128 * 8);
+    p.stats_part = cv.take<double>(STATS_PART_DOUBLES + sizeof(EpisodeLog) / sizeof(double));  // + episode_log(p)
     p.prof = cv.take<unsigned long long>(B * 16);
     p.obs_hdr = cv.take<ssb_obs_hdr>(B);
     p.obs_nodes = cv.take<float>(B * d.Sc * 3);
@@ -442,6 +480,7 @@ int ssb_create(const ssb_config *cfg, const ssb_bank *bk, int device, void *work
     CUDA_TRY(cudaMemset(p.stats, 0, sizeof(ssb_stats) * (size_t)p.B));
     CUDA_TRY(cudaMemset(p.prof, 0, sizeof(unsigned long long) * 16 * (size_t)p.B));
     CUDA_TRY(cudaMemset(p.obs_hdr, 0, sizeof(ssb_obs_hdr) * (size_t)p.B));
+    CUDA_TRY(cudaMemset(episode_log(p), 0, sizeof(EpisodeLog)));  // no episode log attached
     CUDA_TRY(cudaStreamCreateWithFlags(&env->own_stream, cudaStreamNonBlocking));
     CUDA_TRY(cudaEventCreateWithFlags(&env->ev, cudaEventDisableTiming));
     CUDA_TRY(cudaEventCreateWithFlags(&env->ev_last, cudaEventDisableTiming));
@@ -517,7 +556,16 @@ int ssb_i_step_launch(ssb_env *env, const int32_t *stage_idx, const int32_t *num
         k_step<2><<<env->grid, WARPS_PER_CTA * 32, 0, s>>>(env->p, stage_idx, num_exec, mask, max_events, ar, ss, next_a,
                                                            next_n, dyn);
     CUDA_TRY(cudaGetLastError());
+    if (const int rc_ = ssb_i_episode_log_launch(env, s)) return rc_;
     SSB_MARK(env, s);
+    return SSB_OK;
+}
+
+int ssb_i_episode_log_launch(ssb_env *env, cudaStream_t s)
+{
+    if (!env->elog.cur) return SSB_OK;
+    k_episode_log<<<env->grid, WARPS_PER_CTA * 32, 0, s>>>(env->p);
+    CUDA_TRY(cudaGetLastError());
     return SSB_OK;
 }
 
@@ -681,6 +729,7 @@ int ssb_rollout_fair_traj(ssb_env *env, int32_t num_decisions, int32_t dynamic_p
         k_rollout_fair<2><<<env->grid, WARPS_PER_CTA * 32, 0, (cudaStream_t)stream>>>(
             env->p, num_decisions, dynamic_partition, auto_reset, seed_step, traj);
     CUDA_TRY(cudaGetLastError());
+    if (const int rc_ = ssb_i_episode_log_launch(env, (cudaStream_t)stream)) return rc_;
     SSB_MARK(env, stream);
     return SSB_OK;
 }
@@ -697,6 +746,7 @@ int ssb_rollout_fair_async(ssb_env *env, int32_t max_decisions, double rollout_d
         k_rollout_fair_async<2><<<env->grid, WARPS_PER_CTA * 32, 0, (cudaStream_t)stream>>>(
             env->p, max_decisions, rollout_duration, dynamic_partition, seed_step, traj, num_steps, elapsed);
     CUDA_TRY(cudaGetLastError());
+    if (const int rc_ = ssb_i_episode_log_launch(env, (cudaStream_t)stream)) return rc_;
     SSB_MARK(env, stream);
     return SSB_OK;
 }
@@ -788,9 +838,25 @@ int ssb_reset_stats(ssb_env *env, void *stream)
 {
     if (!env) return SSB_E_INVALID;
     SSB_ON_DEVICE(env);
-    k_zero_stats<<<(env->p.B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(env->p.stats, env->p.B);
+    k_zero_stats<<<(env->p.B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(env->p.stats, env->p.B, env->elog.cur);
     CUDA_TRY(cudaGetLastError());
     SSB_MARK(env, stream);
+    return SSB_OK;
+}
+
+int ssb_attach_episode_log(ssb_env *env, ssb_episode *episodes, int32_t capacity, double *job_durations,
+                           int32_t window, ssb_episode_cursor *cursors, void *stream)
+{
+    if (!env) return SSB_E_INVALID;
+    if (cursors && (capacity < 0 || window < 0 || !episodes != (capacity == 0) || !job_durations != (window == 0)))
+        return SSB_E_INVALID;
+    SSB_ON_DEVICE(env);
+    ssb_i_drop_decision_graph(env);  // like the other setters: the next Decima rollout captures its decision again
+    const EpisodeLog L = cursors ? EpisodeLog{episodes, job_durations, cursors, capacity, window} : EpisodeLog{};
+    k_attach_episode_log<<<(env->p.B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(env->p, L);
+    CUDA_TRY(cudaGetLastError());
+    SSB_MARK(env, stream);
+    env->elog = L;
     return SSB_OK;
 }
 

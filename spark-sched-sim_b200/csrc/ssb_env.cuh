@@ -143,6 +143,7 @@ struct ssb_env {
     // Decima policy unit only (ssb_policy.cu): the simulator kernels never see these
     uint32_t *pol_streams;  // [B] policy sampling stream of every env (ssb_set_policy_streams), in the workspace
     RolloutStore store;     // ssb_decima_attach_rollout_store
+    ssb::EpisodeLog elog;   // host copy of what ssb_attach_episode_log attached (elog.cur == nullptr: none)
 };
 
 // ---- internal entry points across the units (C linkage like the public ones; not exported through include/ssb.h)
@@ -151,6 +152,9 @@ extern "C" {
 int ssb_i_step_launch(ssb_env *env, const int32_t *stage_idx, const int32_t *num_exec, const uint8_t *mask,
                       int32_t max_events, int32_t *next_a, int32_t *next_n, int dyn, cudaStream_t s,
                       int force_autoreset, uint64_t force_seed_step);
+// after a launch that steps the envs: the episode log's records and window entries of that launch (no-op unless a log is
+// attached; stream-ordered behind the launch)
+int ssb_i_episode_log_launch(ssb_env *env, cudaStream_t s);
 // ssb_policy.cu
 int ssb_i_decima_obs(ssb_env *env, cudaStream_t s);  // the observation adapter kernel
 void ssb_i_policy_carve(Carver &cv, const ssb_config &c, const Dims &d, ssb::Params &p, uint32_t **pol_streams);

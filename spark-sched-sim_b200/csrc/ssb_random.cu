@@ -72,6 +72,7 @@ int ssb_rollout_random(ssb_env *env, int32_t num_decisions, int32_t auto_reset, 
         k_rollout_random<2><<<env->grid, WARPS_PER_CTA * 32, 0, (cudaStream_t)stream>>>(env->p, num_decisions, auto_reset,
                                                                                         seed_step, traj);
     CUDA_TRY(cudaGetLastError());
+    if (const int rc_ = ssb_i_episode_log_launch(env, (cudaStream_t)stream)) return rc_;
     SSB_MARK(env, stream);
     return SSB_OK;
 }
@@ -88,6 +89,7 @@ int ssb_rollout_random_async(ssb_env *env, int32_t max_decisions, double rollout
         k_rollout_random_async<2><<<env->grid, WARPS_PER_CTA * 32, 0, (cudaStream_t)stream>>>(
             env->p, max_decisions, rollout_duration, seed_step, traj, num_steps, elapsed);
     CUDA_TRY(cudaGetLastError());
+    if (const int rc_ = ssb_i_episode_log_launch(env, (cudaStream_t)stream)) return rc_;
     SSB_MARK(env, stream);
     return SSB_OK;
 }

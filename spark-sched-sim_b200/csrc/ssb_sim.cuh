@@ -767,6 +767,65 @@ struct Sim {
         jb[j].sched = 0;
         jb[j].t_completed = h->wall_time;
     }
+    // ssb_attach_episode_log, whole warp: job_duration_buff.append(t_completed - t_arrival) (:697) for the completions
+    // of the live episode not in the env's window yet, by completion time; equal times by job id (the facade's order,
+    // env.py; the reference's is event order).  Runs via log_launch_w after a launch and at the top of reset_w, so
+    // the window is current whenever a caller can read it; the event loop writes nothing for it.
+    __device__ SSB_RARE void log_job_durations_w()
+    {
+        if (lane == 0) {
+            const EpisodeLog &L = *episode_log(p);
+            ssb_episode_cursor &c = L.cur[b];
+            const int n = h->n_completed, na = h->next_arrival;
+            long long k = c.jobs_completed;
+            for (int todo = n - c.logged; todo > 0; todo--) {  // the earliest completion not logged yet, repeatedly
+                int best = -1;
+                double bt = 0.0;
+                for (int j = 0; j < na; j++)
+                    if (jb[j].state == JOB_COMPLETED && !jb[j].logged && (best < 0 || jb[j].t_completed < bt)) {
+                        best = j;
+                        bt = jb[j].t_completed;
+                    }
+                if (best < 0) break;
+                jb[best].logged = 1;
+                if (L.window > 0)
+                    L.win[(size_t)b * L.window + (size_t)(k % L.window)] = __dsub_rn(bt, jb[best].t_arrival);
+                k++;
+            }
+            c.jobs_completed = k;
+            c.logged = n;
+        }
+        __syncwarp();
+    }
+    // ssb_attach_episode_log, lane 0: the record of an episode whose last observation reports terminated or truncated
+    // (observe_w's test), once (`ended`).  Frozen envs record nothing.  Reached only through log_launch_w, where the
+    // state is still the one the ending step left: k_episode_log after a launch, and reset_w before it wipes it.
+    // The sums run serially in job-index order, so that a host loop restates them bit for bit.
+    __device__ SSB_RARE void log_episode_end(bool terminated, int episode)
+    {
+        const EpisodeLog &L = *episode_log(p);
+        ssb_episode_cursor &c = L.cur[b];
+        const double wall = h->wall_time;
+        const bool truncated = wall >= h->time_limit;
+        if (c.ended || h->error || !(terminated || truncated)) return;
+        const int na = h->next_arrival;
+        double jt = 0.0, sd = 0.0;
+        for (int j = 0; j < na; j++) {
+            const double ta = jb[j].t_arrival, tc = jb[j].t_completed;
+            jt = __dadd_rn(jt, __dsub_rn(fmin(tc, wall), ta));
+            if (jb[j].state == JOB_COMPLETED) sd = __dadd_rn(sd, __dsub_rn(tc, ta));
+        }
+        ssb_episode e;
+        e.seed = h->seed; e.wall_time = wall; e.time_limit = h->time_limit; e.job_time = jt; e.sum_job_duration = sd;
+        e.decisions = (int32_t)(stats->decisions - c.decisions0);
+        e.jobs_arrived = na; e.jobs_completed = h->n_completed;
+        e.flags = (terminated ? 1 : 0) | (truncated ? 2 : 0);
+        e.episode = episode; e.pad = 0;
+        const long long k = c.episodes;
+        if (L.cap > 0) L.rec[(size_t)b * L.cap + (size_t)(k % L.cap)] = e;
+        c.episodes = k + 1;
+        c.ended = 1;
+    }
     __device__ void handle_task_completion(int e, int j, int s)  // :452-483
     {
         StageRec &r = st[jb[j].node_base + s];
@@ -1797,8 +1856,21 @@ struct Sim {
     }
 
     // ------------------------------------------------------------ reset() (:127-186)
+    // ssb_attach_episode_log, whole warp: what the log still lacks of the env's episode -- its record if it has ended,
+    // the completions not yet in the window.  The simulator's event and decision loops do not call it: the entry points
+    // launch k_episode_log after every kernel that steps the envs, and reset_w calls it before it wipes an episode.
+    // `counted`: reset_count already counts the next episode (an auto-reset increments it before reset_w).
+    __device__ SSB_RARE void log_launch_w(bool counted = false)
+    {
+        if (lane == 0) log_episode_end(h->done != 0, h->reset_count - (counted ? 2 : 1));
+        log_job_durations_w();
+    }
+
     __device__ SSB_RARE void reset_w(uint64_t seed, double time_limit)
     {
+        // an episode a fused rollout ended in this launch, before it is wiped.  (Only auto-resets get here with one: the
+        // launch that ended an episode records it, and an explicit reset abandons a live one, which records nothing.)
+        if (episode_log(p)->cur) log_launch_w(true);
         const int Jc = p.Jc;
         int n_jobs = 0, err = 0;
         const bool trace = h->trace_jobs > 0;
@@ -1858,6 +1930,12 @@ struct Sim {
             H.hist_n = 0;
             H.obs_owed = 0;
             H.n_obs_nodes = 0; H.n_obs_edges = 0;  // (the arrivals below add their jobs)
+            if (ssb_episode_cursor *cur = episode_log(p)->cur) {  // the log's cursor: a new episode (a refused reset starts none)
+                ssb_episode_cursor &c = cur[b];
+                c.decisions0 = stats->decisions;
+                c.ended = err ? 1 : 0;
+                c.logged = 0;  // (the jobs' flags are cleared below)
+            }
         }
         __syncwarp();
         if (h->error) {
@@ -1883,7 +1961,7 @@ struct Sim {
                 if (p.b_parent[J.ts_base + s] == 0) fr |= bit64(s);  // job.py:93-111 in-degree 0
             J.frontier = fr;
             J.n_obs_edges = (int16_t)(p.b_edge_base[t + 1] - p.b_edge_base[t]);
-            J.sat = 0; J.sched = 0; J.selected = 0;
+            J.sat = 0; J.sched = 0; J.selected = 0; J.logged = 0;
             J.n_local = 0; J.supply = 0; J.commit_from = 0; J.sat_count = 0; J.state = JOB_PENDING;
         }
         __syncwarp();

@@ -69,7 +69,8 @@ struct __align__(16) JobRec {  // job.py:12-40 + tracker counters keyed by the j
     uint8_t sat_count;    // saturated_stage_count
     uint8_t state;
     int16_t n_obs_edges;  // template edges with both ends in `active`: the job's edges in the observation
-    uint8_t pad[4];
+    uint8_t logged;       // the episode log's window holds this job's duration (set by Sim::log_job_durations_w)
+    uint8_t pad[3];
 };
 static_assert(sizeof(JobRec) == 96, "JobRec layout");
 
@@ -117,6 +118,14 @@ struct __align__(16) EnvHdr {
 };
 static_assert(sizeof(EnvHdr) == 160, "EnvHdr layout");
 
+// The buffers of ssb_attach_episode_log (caller-owned device memory)
+struct EpisodeLog {
+    ssb_episode *rec;         // [B][cap] ring of finished episodes (nullptr when cap == 0)
+    double *win;              // [B][window] ring of completed-job durations (nullptr when window == 0)
+    ssb_episode_cursor *cur;  // [B]
+    int32_t cap, window;
+};
+
 // Everything a kernel needs, passed by value.
 struct Params {
     int B, E, Jc, Sc, Mc, TAB, RT, P, Cc, max_stages;
@@ -151,7 +160,7 @@ struct Params {
     LogRow *log;       // [B][log_cap]
     HistRow *hist;     // [B][hist_cap] executor history (only with ssb_config.history_capacity > 0)
     ssb_stats *stats;  // [B]
-    double *stats_part;  // [128][8] partial sums of ssb_collect_stats
+    double *stats_part;  // [128][8] partial sums of ssb_collect_stats, then the episode log's descriptor (episode_log)
     unsigned long long *prof;  // [B][16] cycle counters per phase (written only when built with -DSSB_PROFILE)
     // observation slabs
     ssb_obs_hdr *obs_hdr;
@@ -202,5 +211,16 @@ struct Params {
     int32_t *as_any;                // [1] envs still taking part
     int lvl_cap;
 };
+
+// The partial sums of ssb_collect_stats ([STATS_BLOCKS][8]) and, right after them in the same workspace region, the
+// descriptor of the log ssb_attach_episode_log attached (cur == nullptr: none).  Reached through p.stats_part so that
+// Params keeps its layout: the simulator kernels copy Params to local memory, and a new field reshuffles that copy and
+// the registers of the whole fused rollout kernel.
+constexpr int STATS_BLOCKS = 128;
+constexpr int STATS_PART_DOUBLES = STATS_BLOCKS * 8;
+__host__ __device__ inline EpisodeLog *episode_log(const Params &p)
+{
+    return reinterpret_cast<EpisodeLog *>(p.stats_part + STATS_PART_DOUBLES);
+}
 
 }  // namespace ssb

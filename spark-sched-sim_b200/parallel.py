@@ -92,8 +92,15 @@ def rollout_summary(sum_job_time: float, sum_wall_time: float, num_completed: fl
 
 def stats_from_sums(vec) -> dict:
     """The reference's per-iteration statistics (trainer.py:310-320 averages the workers' collect_stats dicts)
-    from the (all-reduced) ssb_collect_stats vector."""
+    from the (all-reduced) ssb_collect_stats vector.  With an episode log attached ([7] > 0: envs that have a
+    completed job in their window), avg_job_duration is the mean over those envs of their window's mean -- the
+    trainer's mean over workers of env.avg_job_duration (the last 200 completions, across resets); otherwise the
+    mean duration of the jobs completed in the live episodes."""
     v = [float(x) for x in (vec.tolist() if hasattr(vec, "tolist") else vec)]
     n = max(v[1], 1.0)
+    if len(v) > 7 and v[7] > 0:
+        avg_dur = v[6] / v[7] * 1e-3
+    else:
+        avg_dur = (v[4] / v[2] * 1e-3) if v[2] else float("nan")
     return {"avg_num_jobs": v[0] / n, "num_completed_jobs": v[2] / n, "num_job_arrivals": v[3] / n,
-            "avg_job_duration": (v[4] / v[2] * 1e-3) if v[2] else float("nan")}
+            "avg_job_duration": avg_dur}
